@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the phase-1 hot path (BASELINE.json metric: phase-1 contribute points/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--curve C]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--curve C] [--dump-outputs DIR]
 
 One *step* = Phase1::computation over ONE chunk of the configuration BASELINE.json names for a
 single B200: BLS12-377, 2^20 powers, chunk size 2^16 (262 145 points: 196 608 G1 + 65 537 G2),
@@ -28,6 +28,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (it may be read-only)
 
 CURVE_BITS = {"bls12_377": (12, 253), "bw6_761": (24, 377), "mnt4_753": (24, 753), "mnt6_753": (24, 753)}
 G2_DEG = {"bls12_377": 2, "bw6_761": 1, "mnt4_753": 2, "mnt6_753": 3}
@@ -129,6 +130,42 @@ def declared_work_per_point(curve: str, group: int):
         nw = (bits + 2 + 3) // 4
         terms += [(4 * (nw - 1), dbl), (nw * 15.0 / 16.0, step)]
     return comb(*terms)
+
+
+VECTOR_NAMES = ("tau_powers_g1", "tau_powers_g2", "alpha_tau_powers_g1", "beta_tau_powers_g1", "beta_g2")
+VECTOR_GROUPS = (0, 1, 0, 0, 1)
+DUMP_BUDGET = 64 * 10 ** 6
+
+
+def accumulator_vectors(buf, sz, es, compressed):
+    """Splits an accumulator or a contribution (64-byte hash slot first) into its five point vectors:
+    [(name, uint8 array of shape (points, point bytes))]."""
+    counts = (sz["g1_count"], sz["other_count"], sz["other_count"], sz["other_count"], 1)
+    out, off = [], 64
+    for name, cnt, g in zip(VECTOR_NAMES, counts, VECTOR_GROUPS):
+        pb = es[("g1" if g == 0 else "g2") + ("_c" if compressed else "_u")]
+        out.append((name, buf[off:off + cnt * pb].reshape(cnt, pb)))
+        off += cnt * pb
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: writes every (name, uint8 array of shape (rows, bytes per row)) as out_dir/<name>.npy in float32, one
+    byte per element, so that two builds can be compared output for output.  When the arrays together would exceed
+    DUMP_BUDGET bytes, each keeps the same fraction of its rows (at least one), chosen with a fixed seed, and the kept row
+    indices go to out_dir/<name>_rows.npy (float64)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    full = sum(a.size * 4 for _, a in arrays)
+    sampled = full > DUMP_BUDGET - 4096 * len(arrays)
+    frac = (DUMP_BUDGET - 8192 * len(arrays)) / sum(a.size * 4 + a.shape[0] * 8 for _, a in arrays) if sampled else 1.0
+    rng = np.random.default_rng(20)
+    for name, a in arrays:
+        if sampled:
+            rows = np.sort(rng.choice(a.shape[0], max(1, int(a.shape[0] * frac)), replace=False))
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
 
 
 def macs_per_fq_sqr(limbs: int) -> int:
@@ -281,6 +318,7 @@ def run_phase2(args, rank, world, local_rank):
     barrier()
     ms = run_steps(step, args.steps)
     barrier()
+    last_out = d_out.cpu().numpy() if args.dump_outputs and rank == 0 else None
     launches = sum(v["launches"] for v in sso.profile_read().values()) // max(1, args.steps)
     sso.profile_reset(); sso.profile_enable(2)
     run_steps(step, args.steps)
@@ -314,6 +352,8 @@ def run_phase2(args, rank, world, local_rank):
                              "fq_muls_per_point": round(declared_fq_muls_per_point(name, 0), 1),
                              "kernels": {kk: {"launches": v["launches"], "ms_total": round(v["ms"], 3)} for kk, v in prof.items() if v["launches"]}},
                 "clocks": sampler.summary()}
+        if last_out is not None:
+            dump_outputs(args.dump_outputs, [("scaled_query_g1", last_out.reshape(n, es["g1_u"]))])
         os.write(json_fd, (json.dumps(line) + "\n").encode())
     if dist is not None:
         dist.destroy_process_group()
@@ -461,6 +501,11 @@ def run_verify_transcript(args, rank, world, local_rank):
             dist.all_reduce(vals, op=dist.ReduceOp.MAX)
         stats = sso.dist_stats()
         final_hash = open(f("final.hash"), "rb").read().hex() if rank == 0 else None
+        if args.dump_outputs and rank == 0:
+            import numpy as np
+            final = np.fromfile(f("final"), dtype=np.uint8)
+            dumped = [("final_hash", np.frombuffer(bytes.fromhex(final_hash), dtype=np.uint8).reshape(1, 64))]
+            dump_outputs(args.dump_outputs, dumped + accumulator_vectors(final, full, sso.phase1.curve_sizes(name), False))
     finally:
         barrier()
         if rank == 0:
@@ -501,6 +546,9 @@ def main():
     ap.add_argument("--query-log", type=int, default=20, help="phase2 workload: log2 of the query length")
     ap.add_argument("--batch-log", type=int, default=None, help="log2 of Phase1Parameters::batch_size (default: the chunk size)")
     ap.add_argument("--lanes", type=int, default=3, help="verify_transcript workload: chunks in flight per rank")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (rank 0) as DIR/<name>.npy, float32, "
+                         "at most 64 MB in all; the inputs are the same from run to run, so two builds can be compared")
     args = ap.parse_args()
     if args.batch_log is None:
         args.batch_log = args.chunk_log
@@ -576,17 +624,9 @@ def main():
     sso.contribute_dev(p, d_gen, d_resp, *prev, check=sso.CHECK_NO, device=dev)
     d_ch = torch.empty(acc, dtype=torch.uint8, device="cuda")
     d_ch[:64] = d_gen[:64]
-    offs_u = [64]
-    offs_c = [64]
-    counts = (sz["g1_count"], sz["other_count"], sz["other_count"], sz["other_count"], 1)
-    groups = (0, 1, 0, 0, 1)
-    for cnt, g in zip(counts, groups):
-        offs_u.append(offs_u[-1] + cnt * (es["g1_u"] if g == 0 else es["g2_u"]))
-        offs_c.append(offs_c[-1] + cnt * (es["g1_c"] if g == 0 else es["g2_c"]))
-    for i in range(5):
-        if counts[i]:
-            sso.reencode(args.curve, groups[i], d_resp[offs_c[i]:offs_c[i + 1]], counts[i], d_ch[offs_u[i]:offs_u[i + 1]],
-                         check=sso.CHECK_NO, subgroup_check=False, device=dev)
+    for g, (_, src), (_, dst) in zip(VECTOR_GROUPS, accumulator_vectors(d_resp, sz, es, True), accumulator_vectors(d_ch, sz, es, False)):
+        if src.shape[0]:
+            sso.reencode(args.curve, g, src, src.shape[0], dst, check=sso.CHECK_NO, subgroup_check=False, device=dev)
     del d_gen
     h_ch = torch.empty(acc, dtype=torch.uint8).pin_memory()
     h_ch.copy_(d_ch)
@@ -626,6 +666,7 @@ def main():
     barrier()
     ms_total = run_steps(step_dev, args.steps, True)
     barrier()
+    last_resp = d_resp.cpu().numpy() if args.dump_outputs and rank == 0 else None
     launches_total = sum(v["launches"] for v in sso.profile_read().values())
     # ---- roofline pass: the same steps with every kernel timed by CUDA events on its launching stream and
     # the two streams of a call serialised, so that each kernel's time is its time alone on the GPU
@@ -851,6 +892,8 @@ def main():
     if not args.no_cpu_baseline:
         cb, _ = cpu_reference_run(args.curve, args.power, args.chunk_log, 1, 0, 12.0)
         line["cpu_baseline"] = cb
+    if last_resp is not None:
+        dump_outputs(args.dump_outputs, accumulator_vectors(last_resp, sz, es, True))
     emit(line)
     if dist is not None:
         dist.destroy_process_group()
