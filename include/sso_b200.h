@@ -327,6 +327,24 @@ int32_t sso_p2_verify_file(uint32_t curve, const char* challenge_fn, const char*
                            const char* new_challenge_hash_fn, uint32_t subgroup_check_mode, uint32_t verify_full, int device, char* err,
                            size_t errcap);
 
+/* Radix-2 group FFT of 2^log_n points of one group over the scalar field's two-adic domain (ark-poly Radix2EvaluationDomain
+ * fft / ifft applied to curve points, the primitive of phase2_cli::prepare_phase2, reference
+ * src/bin/intermediate_transform.rs:213-226).  inverse = 0: out_i = sum_j w^(ij) in_j; inverse = 1: out_i = 2^-log_n sum_j w^(-ij) in_j,
+ * natural order, w = GENERATOR^((r - 1) / 2^log_n).  log_n is at most the 2-adicity of Fr and 24.  d_out may equal d_in. */
+int32_t sso_group_fft_dev(uint32_t curve, uint32_t group, const void* d_in, uint32_t in_compressed, uint32_t log_n, uint32_t inverse,
+                          void* d_out, uint32_t out_compressed, int device, char* err, size_t errcap);
+/* phase2_cli::prepare_phase2 (reference src/bin/intermediate_transform.rs:213-226) on host buffers: a Full-mode Groth16 accumulator
+ * (uncompressed) -> the Lagrange-basis Groth16Params of phase2_size = m points (a power of two, m <= 2^power; MNT6-753: m <= 2^15):
+ * alpha_g1 | beta_g1 | beta_g2 | coeffs_g1[m] | coeffs_g2[m] | alpha_coeffs_g1[m] | beta_coeffs_g1[m] | h_g1[m - 1], uncompressed.
+ * Every accumulator element read must be non-zero, on the curve and in the subgroup (SSO_E_INPUT otherwise).
+ * *out_len receives the size of the output; SSO_E_ARG (with the size) when out_cap is too small. */
+int32_t sso_p2_prepare_buf(const sso_p1_params_t* p, const uint8_t* accumulator, size_t len, uint64_t phase2_size, uint8_t* out, size_t out_cap,
+                           size_t* out_len, int device, char* err, size_t errcap);
+/* phase2_cli::prepare_phase2(phase2_filename, response_filename, phase2_size, parameters), argument for argument; the output must not
+ * exist (SSO_E_IO) and is only renamed into place when the call succeeded. */
+int32_t sso_p2_prepare_file(const char* phase2_fn, const char* response_fn, uint64_t phase2_size, const sso_p1_params_t* p, int device,
+                            char* err, size_t errcap);
+
 /* setup_utils::calculate_hash (reference src/utils.rs:618-623): Blake2b-512, unkeyed. Host only. */
 int32_t sso_blake2b_512(const uint8_t* data, size_t len, uint8_t out[64]);
 

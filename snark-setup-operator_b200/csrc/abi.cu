@@ -7,6 +7,7 @@
 #include "flows.cuh"
 #include "files.cuh"
 #include "p2.cuh"
+#include "p2prep.cuh"
 #include <memory>
 #include <thread>
 #include <mutex>
@@ -1448,6 +1449,81 @@ int32_t sso_p2_verify_file(uint32_t curve, const char* challenge_fn, const char*
   if ((rc = write_small(small, new_challenge_hash_fn, h, 64, err, errcap))) return fail(rc);
   if ((rc = out.commit(err, errcap))) return fail(rc);
   return commit_small(small, err, errcap);
+}
+
+// ---------------------------------------------------------------------------------------------
+// prepare_phase2 (p2prep.cuh)
+// ---------------------------------------------------------------------------------------------
+// Radix-2 group FFT over the scalar field's two-adic domain — the primitive of phase2_cli::prepare_phase2
+// (ark-poly Radix2EvaluationDomain::ifft / fft applied to curve points, reference src/bin/intermediate_transform.rs:213-226).
+int32_t sso_group_fft_dev(uint32_t curve, uint32_t group, const void* d_in, uint32_t in_compressed, uint32_t log_n, uint32_t inverse,
+                          void* d_out, uint32_t out_compressed, int device, char* err, size_t errcap) {
+  const CurveOps* ops = ops_for(curve);
+  FftDomain d;
+  if (!ops || !fft_domain(curve, d)) { set_err(err, errcap, "unknown curve %u", curve); return SSO_E_ARG; }
+  Ctx c(err, errcap);
+  int rc = c.init(device);
+  if (rc) return rc;
+  if (group > 1 || !d_in || !d_out) { set_err(err, errcap, "unknown group %u or null buffer", group); return SSO_E_ARG; }
+  uint32_t* d_status;
+  if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
+  CurveSizes cs;
+  curve_sizes(curve, cs);
+  const uint8_t* src = (const uint8_t*)d_in;
+  if (in_compressed && log_n <= 24) {
+    uint8_t* d_u;
+    const uint64_t n = 1ull << log_n;
+    if ((rc = c.alloc((void**)&d_u, n * point_size(cs, group, 0)))) return rc;
+    if ((rc = ops->reencode(c, 0, group, src, 1, n, d_u, 0, CHECK_NO, 0, nullptr, d_status, err, errcap))) return rc;
+    src = d_u;
+  }
+  std::vector<uint8_t> minv;
+  if (inverse) minv = fft_inv_size(d, log_n, ops->fr_bytes);
+  if ((rc = ops->group_fft(c, 0, group, src, log_n, inverse ? d.root_inv : d.root, d.two_adicity, inverse ? minv.data() : nullptr,
+                           (uint8_t*)d_out, out_compressed, d_status, err, errcap))) return rc;
+  if ((rc = sync_all(c, err, errcap))) return rc;
+  return check_status(c, d_status, "group FFT input", err, errcap);
+}
+
+// phase2_cli::prepare_phase2 on host buffers (reference src/bin/intermediate_transform.rs:213-226): a Full-mode accumulator
+// (uncompressed) -> the Lagrange-basis Groth16Params of size phase2_size.  *out_len receives the size; SSO_E_ARG with the needed size
+// in *out_len when out_cap is too small.
+int32_t sso_p2_prepare_buf(const sso_p1_params_t* p, const uint8_t* accumulator, size_t len, uint64_t phase2_size, uint8_t* out, size_t out_cap,
+                           size_t* out_len, int device, char* err, size_t errcap) {
+  if (out_len) *out_len = 0;
+  P1Layout L;
+  FftDomain d;
+  int log_m;
+  int rc = p2prep_check(p, phase2_size, L, d, log_m, err, errcap);
+  if (rc) return rc;
+  if (!out_len) { set_err(err, errcap, "null out_len"); return SSO_E_ARG; }
+  if (!accumulator || len != L.acc_size) { set_err(err, errcap, "accumulator is %zu bytes, the parameters give %llu", len, (unsigned long long)L.acc_size); return SSO_E_ARG; }
+  const size_t need = p2prep_size(L.cs, phase2_size);
+  *out_len = need;
+  if (!out || out_cap < need) { set_err(err, errcap, "output buffer too small: %zu bytes needed", need); return SSO_E_ARG; }
+  Ctx c(err, errcap);
+  if ((rc = c.init(device, 2))) return rc;
+  return p2_prepare(c, ops_for(p->curve), L, d, log_m, accumulator, out, err, errcap);
+}
+
+// phase2_cli::prepare_phase2(phase2_filename, response_filename, phase2_size, parameters) — reference
+// src/bin/intermediate_transform.rs:213-226.  The output is created under a temporary name and renamed when the call succeeded.
+int32_t sso_p2_prepare_file(const char* phase2_fn, const char* response_fn, uint64_t phase2_size, const sso_p1_params_t* p, int device,
+                            char* err, size_t errcap) {
+  if (!phase2_fn || !response_fn) { set_err(err, errcap, "null argument"); return SSO_E_ARG; }
+  P1Layout L;
+  FftDomain d;
+  int log_m;
+  int rc = p2prep_check(p, phase2_size, L, d, log_m, err, errcap);
+  if (rc) return rc;
+  MappedFile in, out;
+  if ((rc = in.open_ro(response_fn, err, errcap))) return rc;
+  size_t need = 0;
+  rc = sso_p2_prepare_buf(p, in.p, in.len, phase2_size, nullptr, 0, &need, device, err, errcap);
+  if (rc != SSO_E_ARG || need == 0) return rc ? rc : SSO_E_ARG;
+  if ((rc = out.create(phase2_fn, need, true, err, errcap))) return rc;
+  if ((rc = sso_p2_prepare_buf(p, in.p, in.len, phase2_size, out.p, out.len, &need, device, err, errcap))) return rc;
+  return out.commit(err, errcap);
 }
 
 int32_t sso_imad_peak(int device, int variant, double* macs_per_s, char* err, size_t errcap) {

@@ -56,6 +56,15 @@ struct CurveOps {
   // device time of decoding + checking + the power-ratio MSM of one G2 element relative to one G1 element (measured launch
   // lists, profiles/r2_verify_kernels_*): chunk verification balances its two streams with it
   float verify_g2_weight;
+  // radix-2 group FFT of 2^log_n uncompressed points (Stockham stages, natural order in and out; kernels.cuh body_fft_butterfly).
+  //   root  : host, canonical words of a root of unity of order 2^two_adicity (its inverse for the inverse transform)
+  //   scale : host, canonical Fr bytes multiplying every output (m^-1 of the inverse transform), or null
+  // d_out may be d_x; the input is only read.
+  int (*group_fft)(Ctx& c, int si, uint32_t group, const uint8_t* d_x, uint32_t log_n, const uint32_t* root, uint32_t two_adicity,
+                   const uint8_t* scale, uint8_t* d_out, uint32_t out_compressed, uint32_t* d_status, char* err, size_t errcap);
+  // d_out[j] = d_hi[j] - d_lo[j] for n uncompressed points
+  int (*points_sub)(Ctx& c, int si, uint32_t group, const uint8_t* d_hi, const uint8_t* d_lo, uint64_t n, uint8_t* d_out,
+                    uint32_t out_compressed, char* err, size_t errcap);
 };
 
 template <class Fr>
@@ -509,6 +518,140 @@ inline int run_reencode(Ctx& c, int si, const uint8_t* d_in, uint32_t in_compres
   return SSO_OK;
 }
 
+// ---------------------------------------------------------------------------------------------
+// group FFT (prepare_phase2)
+// ---------------------------------------------------------------------------------------------
+// the root of unity of one Stockham stage, root^(2^squarings), canonical, followed by three canonical ones: the input of
+// k_tau_tables (tau + coefficient slots)
+template <class Fr>
+__global__ void __launch_bounds__(128, 1) k_fft_stage_root(const uint32_t* root_canon, uint32_t squarings, uint32_t* out_canon) {
+  if (blockIdx.x != 0 || threadIdx.x != 0) return;
+  typename Fr::T w = Fr::to_mont(Fr::from_const(root_canon));
+  for (uint32_t i = 0; i < squarings; i++) w = Fr::sqr(w);
+  w = Fr::from_mont(w);
+  for (int i = 0; i < Fr::L; i++) out_canon[i] = w.v[i];
+  for (int k = 1; k <= TAU_COEFF_SLOTS; k++)
+    for (int i = 0; i < Fr::L; i++) out_canon[k * Fr::L + i] = i == 0 ? 1u : 0u;
+}
+// t_j = w^(j & tw_mask) x[j] over one segment: the batch_exp body with the twiddle scalar source (a separate instantiation,
+// so the k_batch_exp code is unchanged)
+template <class G>
+__global__ void __launch_bounds__(128, (G::GROUP == 0 ? SSO_EXP_MIN_BLOCKS_G1 : SSO_EXP_MIN_BLOCKS_G2)) k_fft_twiddle(const __grid_constant__ VecBatch batch,
+                                                    const uint32_t* table, uint32_t tw_mask, uint32_t* jac_out, uint32_t* status) {
+  extern __shared__ __align__(16) unsigned char tree_raw[];
+  block_batch_exp<G, true>(blockIdx.x, batch, 0, table, CHECK_NO, jac_out, status, reinterpret_cast<typename G::F::T*>(tree_raw), tw_mask);
+}
+template <class G>
+__global__ void __launch_bounds__(128, 1) k_fft_butterfly(uint32_t half, uint32_t log_ns, const uint8_t* x, const uint32_t* tw, uint32_t* jac_out) {
+  body_fft_butterfly<G>(blockIdx.x * blockDim.x + threadIdx.x, half, log_ns, x, tw, jac_out);
+}
+template <class G>
+__global__ void __launch_bounds__(128, 1) k_points_sub(uint32_t n, const uint8_t* hi, const uint8_t* lo, uint32_t* jac_out) {
+  body_points_sub<G>(blockIdx.x * blockDim.x + threadIdx.x, n, hi, lo, jac_out);
+}
+
+template <class G>
+inline int run_normalize_other(Ctx& c, int si, const uint32_t* d_jac, uint64_t n, uint8_t* d_out, uint32_t out_compressed) {
+  VecBatch o;
+  memset(&o, 0, sizeof o);
+  o.seg[0].out = d_out; o.seg[0].n = (uint32_t)n; o.nseg = 1; o.total = (uint32_t)n;
+  c.begin(PK_OTHER, si, n);
+  k_normalize_write<G><<<div_up(div_up(n, NORM_BATCH), 128), 128, 0, c.s[si]>>>(o, d_jac, out_compressed);
+  c.end(si);
+  return SSO_OK;
+}
+
+template <class G>
+inline int run_group_fft(Ctx& c, int si, const uint8_t* d_x, uint32_t log_n, const uint32_t* root, uint32_t two_adicity, const uint8_t* scale,
+                         uint8_t* d_out, uint32_t out_compressed, uint32_t* d_status, char* err, size_t errcap) {
+  using F = typename G::F;
+  using Fr = typename G::Fr;
+  using C = SW<G>;
+  if (log_n > two_adicity || log_n > 24) { set_err(err, errcap, "group FFT of 2^%u points: beyond the radix-2 domain (2^%u) or 2^24", log_n, two_adicity < 24 ? two_adicity : 24); return SSO_E_ARG; }
+  const uint64_t n = 1ull << log_n, half = n / 2;
+  cudaStream_t st = c.s[si];
+  int rc;
+  const uint8_t* cur = d_x;
+  uint8_t* buf[2] = {nullptr, nullptr};
+  if (log_n > 0)
+    for (auto& b : buf) if ((rc = c.alloc((void**)&b, n * C::SIZE_U, si))) return rc;
+  if (scale) {
+    // x * m^-1: one shared-scalar pass before the stages (the a-path of a butterfly has no multiplication to fold it into)
+    const uint8_t* coeffs[TAU_COEFF_SLOTS] = {scale, nullptr, nullptr};
+    uint32_t* d_table;
+    if ((rc = run_tau_tables<Fr>(c, si, 0, nullptr, coeffs, &d_table, err, errcap))) return rc;
+    VecBatch b;
+    memset(&b, 0, sizeof b);
+    b.seg[0].in = d_x; b.seg[0].out = log_n ? buf[0] : d_out; b.seg[0].n = (uint32_t)n; b.seg[0].has_coeff = 1; b.seg[0].mode = 1;
+    b.nseg = 1; b.total = (uint32_t)n;
+    if ((rc = run_batch_exp<G>(c, si, b, 0, d_table, log_n ? 0 : out_compressed, CHECK_NO, d_status, err, errcap))) return rc;
+    if (log_n == 0) return SSO_OK;
+    cur = buf[0];
+  } else if (log_n == 0) {
+    return run_reencode<G>(c, si, d_x, 0, 1, d_out, out_compressed, CHECK_NO, 0, nullptr, d_status, err, errcap);
+  }
+  uint32_t *d_root, *d_stage, *d_table, *d_jac, *d_tw;
+  if ((rc = upload_scalar(c, (const uint8_t*)root, (size_t)Fr::L * 4, Fr::L, &d_root, si, err, errcap))) return rc;
+  if ((rc = c.alloc((void**)&d_stage, (size_t)(1 + TAU_COEFF_SLOTS) * Fr::L * 4, si))) return rc;
+  if ((rc = c.alloc((void**)&d_table, (size_t)TAU_TABLE_ELEMS * Fr::L * 4, si))) return rc;
+  if ((rc = c.alloc((void**)&d_jac, n * 3 * F::WORDS * 4, si))) return rc;
+  if ((rc = c.alloc((void**)&d_tw, half * 3 * F::WORDS * 4, si))) return rc;
+  using GC = typename CoopOf<G>::type;
+  bool coop = false;
+  if constexpr (!std::is_void<GC>::value) coop = coop_g2_enabled<GC>();
+  constexpr size_t TREE_BYTES = 16 + 2 * EXP_BLOCK * sizeof(typename F::T);
+  if (TREE_BYTES > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(k_fft_twiddle<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TREE_BYTES));
+  for (uint32_t s = 0; s < log_n; s++) {
+    uint8_t* nxt = s + 1 == log_n ? d_out : (cur == buf[0] ? buf[1] : buf[0]);
+    const uint32_t* tw = nullptr;
+    if (s > 0) {
+      // twiddles of stage s: powers of the root of order 2^(s+1), for the upper half x[n/2 ..)
+      c.begin(PK_OTHER, si, TAU_TABLE_ELEMS);
+      k_fft_stage_root<Fr><<<1, 32, 0, st>>>(d_root, two_adicity - (s + 1), d_stage);
+      k_tau_tables<Fr><<<div_up(TAU_TABLE_ELEMS, 128), 128, 0, st>>>(d_stage, d_stage + Fr::L, 0, d_table);
+      c.end(si);
+      VecBatch b;
+      memset(&b, 0, sizeof b);
+      b.seg[0].in = cur + half * C::SIZE_U; b.seg[0].n = (uint32_t)half; b.nseg = 1; b.total = (uint32_t)half;
+      const uint32_t mask = (1u << s) - 1;
+      c.begin(G::GROUP == 0 ? PK_BATCH_EXP_G1 : PK_BATCH_EXP_G2, si, half);
+      if constexpr (!std::is_void<GC>::value) {
+        if (coop) {
+          if (ExpBlock<GC>::SMEM > 48 * 1024)
+            CUDA_TRY(cudaFuncSetAttribute(k_fft_twiddle<GC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ExpBlock<GC>::SMEM));
+          k_fft_twiddle<GC><<<div_up(half, ExpBlock<GC>::PPB), EXP_BLOCK, ExpBlock<GC>::SMEM, st>>>(b, d_table, mask, d_tw, d_status);
+        }
+      }
+      if (!coop) k_fft_twiddle<G><<<div_up(half, EXP_BLOCK), EXP_BLOCK, TREE_BYTES, st>>>(b, d_table, mask, d_tw, d_status);
+      c.end(si);
+      tw = d_tw;
+    }
+    c.begin(PK_OTHER, si, n);
+    k_fft_butterfly<G><<<div_up(half, 128), 128, 0, st>>>((uint32_t)half, s, cur, tw, d_jac);
+    c.end(si);
+    run_normalize_other<G>(c, si, d_jac, n, nxt, s + 1 == log_n ? out_compressed : 0);
+    cur = nxt;
+  }
+  CUDA_TRY(cudaGetLastError());
+  return SSO_OK;
+}
+
+template <class G>
+inline int run_points_sub(Ctx& c, int si, const uint8_t* d_hi, const uint8_t* d_lo, uint64_t n, uint8_t* d_out, uint32_t out_compressed,
+                          char* err, size_t errcap) {
+  if (n == 0) return SSO_OK;
+  if (n > (1ull << 30)) { set_err(err, errcap, "vector too long"); return SSO_E_ARG; }
+  uint32_t* d_jac;
+  int rc;
+  if ((rc = c.alloc((void**)&d_jac, n * 3 * G::F::WORDS * 4, si))) return rc;
+  c.begin(PK_OTHER, si, n);
+  k_points_sub<G><<<div_up(n, 128), 128, 0, c.s[si]>>>((uint32_t)n, d_hi, d_lo, d_jac);
+  c.end(si);
+  run_normalize_other<G>(c, si, d_jac, n, d_out, out_compressed);
+  CUDA_TRY(cudaGetLastError());
+  return SSO_OK;
+}
+
 template <class G1, class G2, class PP> struct CurveImpl {
   static int same_ratio(Ctx& c, int si, const uint8_t* d_checks, uint64_t n, uint32_t* d_verdicts, char* err, size_t errcap) {
     return run_same_ratio<G1, G2, PP>(c, si, d_checks, n, d_verdicts, err, errcap);
@@ -580,8 +723,22 @@ template <class G1, class G2, class PP> struct CurveImpl {
     set_err(err, errcap, "unknown group %u", group);
     return SSO_E_ARG;
   }
+  static int group_fft(Ctx& c, int si, uint32_t group, const uint8_t* d_x, uint32_t log_n, const uint32_t* root, uint32_t two_adicity,
+                       const uint8_t* scale, uint8_t* d_out, uint32_t out_compressed, uint32_t* d_status, char* err, size_t errcap) {
+    if (group == GROUP_G1) return run_group_fft<G1>(c, si, d_x, log_n, root, two_adicity, scale, d_out, out_compressed, d_status, err, errcap);
+    if (group == GROUP_G2) return run_group_fft<G2>(c, si, d_x, log_n, root, two_adicity, scale, d_out, out_compressed, d_status, err, errcap);
+    set_err(err, errcap, "unknown group %u", group);
+    return SSO_E_ARG;
+  }
+  static int points_sub(Ctx& c, int si, uint32_t group, const uint8_t* d_hi, const uint8_t* d_lo, uint64_t n, uint8_t* d_out,
+                        uint32_t out_compressed, char* err, size_t errcap) {
+    if (group == GROUP_G1) return run_points_sub<G1>(c, si, d_hi, d_lo, n, d_out, out_compressed, err, errcap);
+    if (group == GROUP_G2) return run_points_sub<G2>(c, si, d_hi, d_lo, n, d_out, out_compressed, err, errcap);
+    set_err(err, errcap, "unknown group %u", group);
+    return SSO_E_ARG;
+  }
   static const CurveOps* ops() {
-    static const CurveOps o = {&tau_tables, &batch_exp, &batch_exp_chunk, &reencode, &msm_pairs, &same_ratio, (uint32_t)Pairing<G1, G2, PP>::CHECK_BYTES, &keygen_g1, &keygen_scalars, &hash_to_g2, (uint32_t)G1::Fr::L, &points_sum, &fill_generator, (uint32_t)G1::Fr::NBYTES, {2u * G1::F::WORDS, 2u * G2::F::WORDS}, G2::VERIFY_WEIGHT};
+    static const CurveOps o = {&tau_tables, &batch_exp, &batch_exp_chunk, &reencode, &msm_pairs, &same_ratio, (uint32_t)Pairing<G1, G2, PP>::CHECK_BYTES, &keygen_g1, &keygen_scalars, &hash_to_g2, (uint32_t)G1::Fr::L, &points_sum, &fill_generator, (uint32_t)G1::Fr::NBYTES, {2u * G1::F::WORDS, 2u * G2::F::WORDS}, G2::VERIFY_WEIGHT, &group_fft, &points_sub};
     return &o;
   }
 };

@@ -162,10 +162,12 @@ template <class G> struct ExpTypes {
 };
 
 // staged_src: the thread's serialized input point in shared memory (block_stage_input), or null = read it from global memory
-template <class G>
+// TWIDDLE (group FFT, body_fft_butterfly): the scalar of element j is tau^(j & tw_mask) — the table holds the powers of the
+// stage's root of unity, so each butterfly gets its twiddle without a pow per point; the segment's scalar rule is not read
+template <class G, bool TWIDDLE = false>
 __device__ __forceinline__ typename G::F::T exp_stage_a(uint32_t tid, const VecBatch& b, uint32_t in_compressed, const uint32_t* table,
                                                         uint32_t check, uint32_t* status, typename ExpTypes<G>::State& st,
-                                                        const uint8_t* staged_src = nullptr) {
+                                                        const uint8_t* staged_src = nullptr, uint32_t tw_mask = 0) {
   using C = SW<G>;
   using F = typename G::F;
   using Fr = typename G::Fr;
@@ -186,7 +188,9 @@ __device__ __forceinline__ typename G::F::T exp_stage_a(uint32_t tid, const VecB
     else if (check == CHECK_FULL && !in_compressed && !C::on_curve(p)) { report(status, ST_NOT_ON_CURVE, j, sidx); p.inf = true; }
   }
   uint32_t k[Fr::L];
-  if (sg.mode == 0) {
+  if constexpr (TWIDDLE) {
+    scalar_for_index<Fr>(table, j & tw_mask, tw_mask + 1, false, 0, k);
+  } else if (sg.mode == 0) {
     scalar_for_index<Fr>(table, j, sg.n, sg.has_coeff != 0, sg.coeff_slot, k);
   } else {
     typename Fr::T s = Fr::from_mont(Fr::load(table + (size_t)(769 + sg.coeff_slot) * Fr::L, 1));
@@ -288,9 +292,9 @@ template <class G> struct ExpBlock {
 };
 
 // Cooperative body (coop.cuh): DEG lanes per point.  The tree holds one array of 2 PPB coefficients per role.
-template <class G>
+template <class G, bool TWIDDLE = false>
 __device__ __forceinline__ void block_batch_exp_coop(uint32_t block, const VecBatch& b, const uint32_t* table, uint32_t check,
-                                                     uint32_t* jac_out, uint32_t* status, unsigned char* smem) {
+                                                     uint32_t* jac_out, uint32_t* status, unsigned char* smem, uint32_t tw_mask = 0) {
   using F = typename G::F;
   using CO = Coop<F::DEG>;
   constexpr int PPB = ExpBlock<G>::PPB, TL = ExpBlock<G>::TL;
@@ -299,7 +303,7 @@ __device__ __forceinline__ void block_batch_exp_coop(uint32_t block, const VecBa
   const uint32_t pb = lane_ok ? CO::group_in_block() : 0xffffffffu;
   const uint32_t tid = lane_ok ? block * PPB + pb : 0xffffffffu;       // idle lanes locate nothing and never exchange
   const uint8_t* staged = block_stage_input<G, PPB>(block, b, 0, smem, pb);
-  typename F::T leaf = exp_stage_a<G>(tid, b, 0, table, check, status, st, staged);
+  typename F::T leaf = exp_stage_a<G, TWIDDLE>(tid, b, 0, table, check, status, st, staged, tw_mask);
   __syncthreads();
   if constexpr (G::AFFINE_TABLE) {
     typename F::T* tree = reinterpret_cast<typename F::T*>(smem) + (size_t)(lane_ok ? CO::role() : 0) * 2 * TL;
@@ -318,16 +322,17 @@ __device__ __forceinline__ void block_batch_exp_coop(uint32_t block, const VecBa
   if (lane_ok) exp_stage_c<G>(tid, b, st, leaf, jac_out);
 }
 
-template <class G>
+template <class G, bool TWIDDLE = false>
 __device__ __forceinline__ void block_batch_exp(uint32_t block, const VecBatch& b, uint32_t in_compressed, const uint32_t* table,
-                                                uint32_t check, uint32_t* jac_out, uint32_t* status, typename G::F::T* tree) {
+                                                uint32_t check, uint32_t* jac_out, uint32_t* status, typename G::F::T* tree,
+                                                uint32_t tw_mask = 0) {
   if constexpr (G::F::COOP != 0) {
-    block_batch_exp_coop<G>(block, b, table, check, jac_out, status, reinterpret_cast<unsigned char*>(tree));
+    block_batch_exp_coop<G, TWIDDLE>(block, b, table, check, jac_out, status, reinterpret_cast<unsigned char*>(tree), tw_mask);
   } else {
     typename ExpTypes<G>::State st;
     uint32_t tid = block * EXP_BLOCK + threadIdx.x;
     const uint8_t* staged = block_stage_input<G>(block, b, in_compressed, reinterpret_cast<uint8_t*>(tree));
-    typename G::F::T leaf = exp_stage_a<G>(tid, b, in_compressed, table, check, status, st, staged);
+    typename G::F::T leaf = exp_stage_a<G, TWIDDLE>(tid, b, in_compressed, table, check, status, st, staged, tw_mask);
     __syncthreads();                                                  // the staged bytes are dead: the tree may take the buffer
     if constexpr (G::AFFINE_TABLE) {
       tree[EXP_BLOCK + threadIdx.x] = leaf;
@@ -432,6 +437,60 @@ __device__ __forceinline__ void body_normalize_write(uint32_t tid, const VecBatc
     if (out_compressed) C::write_compressed(out + (size_t)j * C::SIZE_C, a);
     else C::write_uncompressed(out + (size_t)j * C::SIZE_U, a);
   }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Group FFT (prepare_phase2: the Lagrange-basis transform of phase-2 setup): radix-2 Stockham stages, natural order in and out.
+// Stage s (Ns = 2^s) over n points x (uncompressed) takes, for each j < n / 2,
+//   a = x[j],  t = w^(j mod Ns) x[j + n/2]  (w = the root of unity of order 2 Ns; t from the twiddle batch_exp: exp_stage_a
+//   TWIDDLE over the upper half, Jacobian SoA, n / 2 points; stage 0 has only the trivial twiddle 1 and reads x[j + n/2] itself)
+// and writes a + t to o = 2 Ns floor(j / Ns) + (j mod Ns) and a - t to o + Ns (Jacobian SoA, n points) for body_normalize_write.
+// The Jacobian additions are the complete ones: a = t doubles, a = -t and infinity give the identity.
+// ---------------------------------------------------------------------------------------------
+template <class G>
+__device__ __forceinline__ void body_fft_butterfly(uint32_t j, uint32_t half, uint32_t log_ns, const uint8_t* x, const uint32_t* tw,
+                                                   uint32_t* jac_out) {
+  using C = SW<G>;
+  using F = typename G::F;
+  if (j >= half) return;
+  typename C::Affine pa, pb;
+  C::read_uncompressed(x + (size_t)j * C::SIZE_U, pa);
+  typename C::Jac a = C::from_affine(pa), t;
+  if (tw) {
+    t.X = F::load(tw + j, half);
+    t.Y = F::load(tw + (size_t)F::WORDS * half + j, half);
+    t.Z = F::load(tw + (size_t)2 * F::WORDS * half + j, half);
+  } else {
+    C::read_uncompressed(x + ((size_t)j + half) * C::SIZE_U, pb);
+    t = C::from_affine(pb);
+  }
+  const typename C::Jac s = C::add(a, t), d = C::add(a, C::neg(t));
+  const uint32_t ns = 1u << log_ns;
+  const uint32_t o = ((j >> log_ns) << (log_ns + 1)) + (j & (ns - 1));
+  const size_t n = (size_t)2 * half;
+  uint32_t* base = jac_out + o;
+  F::store(base, n, s.X);
+  F::store(base + (size_t)F::WORDS * n, n, s.Y);
+  F::store(base + (size_t)2 * F::WORDS * n, n, s.Z);
+  base += ns;
+  F::store(base, n, d.X);
+  F::store(base + (size_t)F::WORDS * n, n, d.Y);
+  F::store(base + (size_t)2 * F::WORDS * n, n, d.Z);
+}
+
+// h_g1 of prepare_phase2: out[j] = hi[j] - lo[j] (uncompressed inputs) as Jacobian SoA over n points
+template <class G>
+__device__ __forceinline__ void body_points_sub(uint32_t j, uint32_t n, const uint8_t* hi, const uint8_t* lo, uint32_t* jac_out) {
+  using C = SW<G>;
+  using F = typename G::F;
+  if (j >= n) return;
+  typename C::Affine ph, pl;
+  C::read_uncompressed(hi + (size_t)j * C::SIZE_U, ph);
+  C::read_uncompressed(lo + (size_t)j * C::SIZE_U, pl);
+  const typename C::Jac r = C::add(C::from_affine(ph), C::neg(C::from_affine(pl)));
+  F::store(jac_out + j, n, r.X);
+  F::store(jac_out + (size_t)F::WORDS * n + j, n, r.Y);
+  F::store(jac_out + (size_t)2 * F::WORDS * n + j, n, r.Z);
 }
 
 // ---------------------------------------------------------------------------------------------

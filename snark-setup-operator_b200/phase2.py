@@ -7,7 +7,7 @@ from __future__ import annotations
 import ctypes
 
 from ._lib import call
-from .phase1 import CHECK_NO, curve_id, curve_sizes, scalar_bytes
+from .phase1 import CHECK_NO, _dptr, curve_id, curve_sizes, scalar_bytes
 
 
 def scale_queries(curve, queries, n: int, delta_inv: int, in_compressed=False, out_compressed=False, check=CHECK_NO,
@@ -83,3 +83,35 @@ def verify(curve, challenge_filename, challenge_hash_filename, check_input, resp
     call("sso_p2_verify_file", curve_id(curve), challenge_filename.encode(), challenge_hash_filename.encode(), check_input, response_filename.encode(),
          response_hash_filename.encode(), check_output, new_challenge_filename.encode(), new_challenge_hash_filename.encode(), subgroup_check_mode,
          int(verify_full), device)
+
+
+def group_fft(curve, group: int, d_in, log_n: int, d_out, inverse=False, in_compressed=False, out_compressed=False, device=0):
+    """Radix-2 group FFT of 2^log_n points (device buffers: torch uint8 CUDA tensors) over the scalar field's two-adic domain:
+    inverse=False gives out_i = sum_j w^(ij) in_j, inverse=True out_i = 2^-log_n sum_j w^(-ij) in_j, natural order."""
+    call("sso_group_fft_dev", curve_id(curve), group, _dptr(d_in), int(in_compressed), log_n, int(inverse), _dptr(d_out),
+         int(out_compressed), device)
+
+
+def prepare_phase2_buf(parameters, accumulator, phase2_size: int, device=0) -> bytes:
+    """phase2_cli::prepare_phase2 on host buffers: a Full-mode accumulator (uncompressed, `parameters` a Phase1Parameters) ->
+    the Lagrange-basis Groth16Params of phase2_size points (alpha_g1 | beta_g1 | beta_g2 | coeffs_g1 | coeffs_g2 |
+    alpha_coeffs_g1 | beta_coeffs_g1 | h_g1, uncompressed)."""
+    from ._lib import SsoError, lib
+    from .phase1 import _host_ptr
+    ptr, n, keep = _host_ptr(accumulator)
+    need = ctypes.c_size_t(0)
+    err = ctypes.create_string_buffer(512)
+    p = parameters.c_struct()
+    rc = lib().sso_p2_prepare_buf(ctypes.byref(p), ptr, n, phase2_size, None, 0, ctypes.byref(need), device, err, len(err))
+    if rc != -1 or need.value == 0:
+        raise SsoError(rc, err.value.decode("utf-8", "replace"))
+    out = ctypes.create_string_buffer(need.value)
+    call("sso_p2_prepare_buf", ctypes.byref(p), ptr, n, phase2_size, out, len(out), ctypes.byref(need), device)
+    del keep
+    return out.raw
+
+
+def prepare_phase2(phase2_filename, response_filename, phase2_size: int, parameters, device=0):
+    """phase2_cli::prepare_phase2, argument for argument (reference src/bin/intermediate_transform.rs:213-226)."""
+    call("sso_p2_prepare_file", phase2_filename.encode(), response_filename.encode(), phase2_size, ctypes.byref(parameters.c_struct()),
+         device)
