@@ -356,6 +356,15 @@ int32_t sso_imad_peak(int device, int variant, double* macs_per_s, char* err, si
  * little-endian elements of the field's serialized size. field: 0 r253, 1 q377, 2 q761, 3 q4(753), 4 q6(753). */
 int32_t sso_test_field_mul(uint32_t field, const uint8_t* a, const uint8_t* b, uint8_t* out, uint64_t n, int device,
                            char* err, size_t errcap);
+/* Test hook: one field operation per element on raw little-endian Montgomery words, loaded without reduction or range check
+ * and returned as the arithmetic leaves them (csrc/field_probe.cuh).  field: 0 r253, 1 q377, 2 q761, 3 q4(753), 4 q6(753),
+ * 5 q377^2 (u^2 = -5), 6 q4^2 (u^2 = 13), 7 q6^3 (u^3 = 11), 8-10 the same three extensions over 2 / 3 cooperating lanes.
+ * Element i has ops[i] and k[i] (the factor of mad_small_lazy); a, b, out hold n elements of the field's words, coefficient after
+ * coefficient.  ops: 0 mul, 1 add, 2 sub, 3 sqr, 4 neg, 5 inv, 6 dedicated sqr, 7 lex_is_neg, 8 sqrt, 9 reduce_small,
+ * 10 mad_small_lazy(a, k, b), 11 conj, 12 mul_base(a, b.c0), 13 mul_u2, 14 frob_w.  rc[i]: the predicate of ops 7 / 8 (1 = negative,
+ * 1 = root found), 0 otherwise, 0xffffffff for an op the field does not have (out[i] then stays zero). */
+int32_t sso_test_field_op(uint32_t field, const uint32_t* ops, const uint32_t* a, const uint32_t* b, const uint32_t* k, uint32_t* out,
+                          uint32_t* rc, uint64_t n, int device, char* err, size_t errcap);
 
 #ifdef __cplusplus
 }

@@ -90,9 +90,10 @@ def lib() -> ctypes.CDLL:
         L.sso_profile_read.argtypes = [ctypes.POINTER(u64), sz]
         L.sso_imad_peak.argtypes = [i32, i32, ctypes.POINTER(ctypes.c_double), cp, sz]
         L.sso_test_field_mul.argtypes = [u32, u8p, u8p, cp, u64, i32, cp, sz]
+        L.sso_test_field_op.argtypes = [u32, vp, vp, vp, vp, vp, vp, u64, i32, cp, sz]
         for name in ("sso_device_name", "sso_curve_sizes", "sso_p1_sizes", "sso_blake2b_512", "sso_batch_exp_dev",
                      "sso_batch_mul_dev", "sso_reencode_dev", "sso_p1_contribute_dev", "sso_p1_contribute_buf", "sso_imad_peak",
-                     "sso_test_field_mul", "sso_p1_new_challenge_dev", "sso_profile_enable", "sso_profile_reset",
+                     "sso_test_field_mul", "sso_test_field_op", "sso_p1_new_challenge_dev", "sso_profile_enable", "sso_profile_reset",
                      "sso_profile_read", "sso_power_pairs_dev", "sso_merge_pairs_dev", "sso_same_ratio", "sso_p1_keygen",
                      "sso_p1_contribute_seeded_buf", "sso_p1_contribute_file", "sso_p1_verify_chunk_buf", "sso_p1_verify_chunk_file", "sso_points_sum",
                      "sso_p2_scale_queries_buf", "sso_p2_verify_queries_buf", "sso_p1_contribute_many_buf", "sso_p1_verify_chunk_many_buf",

@@ -103,6 +103,10 @@ __global__ void k_imad_probe(uint32_t iters, uint32_t variant, uint32_t seed, ui
 namespace sso {
 ProfSlot g_prof[PK_COUNT];
 std::atomic<int> g_prof_enabled{0};
+
+// field_probe.cu (test-only kernels of sso_test_field_op)
+int run_field_op(Ctx& c, int si, uint32_t field, const uint32_t* d_ops, const uint32_t* d_a, const uint32_t* d_b, const uint32_t* d_k,
+                 uint32_t* d_out, uint32_t* d_rc, uint64_t n, char* err, size_t errcap);
 }  // namespace sso
 
 namespace {
@@ -1584,6 +1588,33 @@ int32_t sso_test_field_mul(uint32_t field, const uint8_t* a, const uint8_t* b, u
   CUDA_TRY(cudaMemcpyAsync(out, d_o, bytes, cudaMemcpyDeviceToHost, c.s[0]));
   if ((rc = sync_all(c, err, errcap))) return rc;
   return check_status(c, d_status, "field element", err, errcap);
+}
+
+int32_t sso_test_field_op(uint32_t field, const uint32_t* ops, const uint32_t* a, const uint32_t* b, const uint32_t* k, uint32_t* out,
+                          uint32_t* rc, uint64_t n, int device, char* err, size_t errcap) {
+  static const uint32_t words[11] = {8, 12, 24, 24, 24, 24, 48, 72, 24, 48, 72};     // per element, by field id
+  if (field > 10) { set_err(err, errcap, "unknown field %u", field); return SSO_E_ARG; }
+  Ctx c(err, errcap);
+  int rc_ = c.init(device);
+  if (rc_) return rc_;
+  const size_t wbytes = n * words[field] * 4, nbytes = n * 4;
+  uint32_t *d_ops, *d_a, *d_b, *d_k, *d_out, *d_rc;
+  if ((rc_ = c.alloc((void**)&d_ops, nbytes))) return rc_;
+  if ((rc_ = c.alloc((void**)&d_a, wbytes))) return rc_;
+  if ((rc_ = c.alloc((void**)&d_b, wbytes))) return rc_;
+  if ((rc_ = c.alloc((void**)&d_k, nbytes))) return rc_;
+  if ((rc_ = c.alloc((void**)&d_out, wbytes))) return rc_;
+  if ((rc_ = c.alloc((void**)&d_rc, nbytes))) return rc_;
+  CUDA_TRY(cudaMemcpyAsync(d_ops, ops, nbytes, cudaMemcpyHostToDevice, c.s[0]));
+  CUDA_TRY(cudaMemcpyAsync(d_a, a, wbytes, cudaMemcpyHostToDevice, c.s[0]));
+  CUDA_TRY(cudaMemcpyAsync(d_b, b, wbytes, cudaMemcpyHostToDevice, c.s[0]));
+  CUDA_TRY(cudaMemcpyAsync(d_k, k, nbytes, cudaMemcpyHostToDevice, c.s[0]));
+  CUDA_TRY(cudaMemsetAsync(d_out, 0, wbytes, c.s[0]));
+  CUDA_TRY(cudaMemsetAsync(d_rc, 0, nbytes, c.s[0]));
+  if ((rc_ = run_field_op(c, 0, field, d_ops, d_a, d_b, d_k, d_out, d_rc, n, err, errcap))) return rc_;
+  CUDA_TRY(cudaMemcpyAsync(out, d_out, wbytes, cudaMemcpyDeviceToHost, c.s[0]));
+  CUDA_TRY(cudaMemcpyAsync(rc, d_rc, nbytes, cudaMemcpyDeviceToHost, c.s[0]));
+  return sync_all(c, err, errcap);
 }
 
 }  // extern "C"

@@ -20,6 +20,7 @@
 #include "../../snark-setup-operator_b200/csrc/msm.cuh"
 #include "../../snark-setup-operator_b200/csrc/pairing.cuh"
 #include "../../snark-setup-operator_b200/csrc/keygen.cuh"
+#include "../../snark-setup-operator_b200/csrc/field_probe.cuh"
 
 using namespace sso;
 
@@ -105,6 +106,34 @@ extern "C" int emul_lazy_probe(int field, int op, const uint32_t* a, const uint3
     case 2: return lazy_probe<Fq761>(op, a, b, k, out);
     case 3: return lazy_probe<Fq4>(op, a, b, k, out);
     case 4: return lazy_probe<Fq6>(op, a, b, k, out);
+  }
+  return -3;
+}
+
+// sso_test_field_op on the CPU: the same body (field_probe.cuh), the same field ids and op codes; a cooperative field runs all
+// its elements on DEG lockstep lane threads
+template <class F, class G> static void field_op_raw(const uint32_t* ops, const uint32_t* a, const uint32_t* b, const uint32_t* k,
+                                                     uint32_t* out, uint32_t* rc, uint64_t n) {
+  if constexpr (F::COOP == 0) {
+    for (uint64_t i = 0; i < n; i++) body_field_op<F, G>((uint32_t)i, ops, a, b, k, out, rc);
+  } else {
+    coop_emu_run(F::DEG, [&](int) { for (uint64_t i = 0; i < n; i++) body_field_op<F, G>((uint32_t)i, ops, a, b, k, out, rc); });
+  }
+}
+extern "C" int emul_field_op_raw(uint32_t field, const uint32_t* ops, const uint32_t* a, const uint32_t* b, const uint32_t* k,
+                                 uint32_t* out, uint32_t* rc, uint64_t n) {
+  switch (field) {
+    case 0: field_op_raw<Fr253, void>(ops, a, b, k, out, rc, n); return 0;
+    case 1: field_op_raw<Fq377, Bls12_377_G1>(ops, a, b, k, out, rc, n); return 0;
+    case 2: field_op_raw<Fq761, Bw6_761_G1>(ops, a, b, k, out, rc, n); return 0;
+    case 3: field_op_raw<Fq4, Mnt4_753_G1>(ops, a, b, k, out, rc, n); return 0;
+    case 4: field_op_raw<Fq6, Mnt6_753_G1>(ops, a, b, k, out, rc, n); return 0;
+    case 5: field_op_raw<Fq377x2, Bls12_377_G2>(ops, a, b, k, out, rc, n); return 0;
+    case 6: field_op_raw<Fq4x2, Mnt4_753_G2>(ops, a, b, k, out, rc, n); return 0;
+    case 7: field_op_raw<Fq6x3, Mnt6_753_G2>(ops, a, b, k, out, rc, n); return 0;
+    case 8: field_op_raw<Bls12_377_G2C::F, Bls12_377_G2C>(ops, a, b, k, out, rc, n); return 0;
+    case 9: field_op_raw<Mnt4_753_G2C::F, Mnt4_753_G2C>(ops, a, b, k, out, rc, n); return 0;
+    case 10: field_op_raw<Mnt6_753_G2C::F, Mnt6_753_G2C>(ops, a, b, k, out, rc, n); return 0;
   }
   return -3;
 }
