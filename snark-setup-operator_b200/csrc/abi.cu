@@ -176,12 +176,57 @@ int single_vector(Ctx& c, const CurveOps* ops, uint32_t group, const uint8_t* d_
   return ops->batch_exp(c, 0, group, b, in_compressed, d_table, out_compressed, check, d_status, err, errcap);
 }
 
-int status_buffer(Ctx& c, uint32_t** d_status, char* err, size_t errcap) {
-  int rc = c.alloc((void**)d_status, STATUS_BYTES);
-  if (rc) return rc;
-  CUDA_TRY(cudaMemsetAsync(*d_status, 0, STATUS_BYTES, c.s[0]));
-  CUDA_TRY(cudaStreamSynchronize(c.s[0]));
+// one vector of points on the device and the checks it is decoded with
+struct PairInput { const uint8_t* d; uint32_t compressed, check, subgroup; };
+
+// Decodes n points to affine and returns on the host the random-linear-combination pair (two uncompressed points):
+// (sum r_i a_i, sum r_i a_{i+1}) over n - 1 terms [power_pairs] when b.d is null, else (sum r_i a_i, sum r_i b_i) [merge_pairs].
+// A point that fails its check is reported as `what`.
+int pair_to_host(Ctx& c, const CurveOps* ops, uint32_t group, size_t usz, uint64_t n, PairInput a, PairInput b, const uint8_t* seed32,
+                 const uint64_t* tweak, uint32_t* d_status, const char* what, uint8_t* pair, char* err, size_t errcap) {
+  int rc;
+  const size_t aff = ops->aff_words[group];
+  uint32_t *d_aff_a, *d_aff_b = nullptr;
+  uint8_t* d_pair;
+  if ((rc = c.alloc((void**)&d_aff_a, n * aff * 4))) return rc;
+  if (b.d && (rc = c.alloc((void**)&d_aff_b, n * aff * 4))) return rc;
+  if ((rc = c.alloc((void**)&d_pair, 2 * usz))) return rc;
+  if ((rc = ops->reencode(c, 0, group, a.d, a.compressed, n, nullptr, 0, a.check, a.subgroup, d_aff_a, d_status, err, errcap))) return rc;
+  if (b.d && (rc = ops->reencode(c, 0, group, b.d, b.compressed, n, nullptr, 0, b.check, b.subgroup, d_aff_b, d_status, err, errcap))) return rc;
+  if ((rc = ops->msm_pairs(c, 0, group, d_aff_a, b.d ? d_aff_b : d_aff_a + aff, b.d ? n : n - 1, seed32, tweak, d_pair, err, errcap))) return rc;
+  if ((rc = sync_all(c, err, errcap))) return rc;
+  if ((rc = check_status(c, d_status, what, err, errcap))) return rc;
+  CUDA_TRY(cudaMemcpy(pair, d_pair, 2 * usz, cudaMemcpyDeviceToHost));
   return SSO_OK;
+}
+
+// batch_exp (mode 0: tau^(first_index + i) [* coeff]) and batch_mul (mode 1: the index-independent scalar `coeff`) of one vector.
+// Vectors longer than the span of one tau table (2^24 indices) are processed in segments, each with its own table base.
+int32_t batch_scalar_dev(uint32_t curve, uint32_t group, const void* d_in, uint32_t in_compressed, uint64_t n, uint64_t first_index,
+                         const uint8_t* tau, const uint8_t* coeff, uint32_t mode, void* d_out, uint32_t out_compressed, uint32_t check_input,
+                         int device, char* err, size_t errcap) {
+  const CurveOps* ops = ops_for(curve);
+  if (!ops || !(mode ? coeff : tau)) { set_err(err, errcap, "unknown curve %u or null scalar", curve); return SSO_E_ARG; }
+  Ctx c(err, errcap);
+  int rc = c.init(device);
+  if (rc) return rc;
+  uint32_t* d_status;
+  if ((rc = status_buffer(c, &d_status, 0, true, err, errcap))) return rc;
+  if (group > 1) { set_err(err, errcap, "unknown group %u", group); return SSO_E_ARG; }
+  std::vector<uint8_t> one(ops->fr_bytes, 0);
+  one[0] = 1;
+  CurveSizes cs;
+  curve_sizes(curve, cs);
+  const uint64_t in_sz = point_size(cs, group, in_compressed), out_sz = point_size(cs, group, out_compressed);
+  const uint64_t SEG = 1ull << 22;
+  for (uint64_t off = 0; off < n; off += SEG) {
+    uint64_t m = n - off < SEG ? n - off : SEG;
+    if ((rc = single_vector(c, ops, group, (const uint8_t*)d_in + off * in_sz, in_compressed, m, mode ? 0 : first_index + off,
+                            mode ? one.data() : tau, coeff, mode, (uint8_t*)d_out + off * out_sz, out_compressed, check_input, d_status,
+                            err, errcap))) return rc;
+  }
+  if ((rc = sync_all(c, err, errcap))) return rc;
+  return check_status(c, d_status, mode ? "batch_mul input" : "batch_exp input", err, errcap);
 }
 
 }  // namespace
@@ -236,54 +281,13 @@ int32_t sso_blake2b_512(const uint8_t* data, size_t len, uint8_t out[64]) {
 int32_t sso_batch_exp_dev(uint32_t curve, uint32_t group, const void* d_in, uint32_t in_compressed, uint64_t n,
                           uint64_t first_index, const uint8_t* tau, const uint8_t* coeff, void* d_out,
                           uint32_t out_compressed, uint32_t check_input, int device, char* err, size_t errcap) {
-  const CurveOps* ops = ops_for(curve);
-  if (!ops || !tau) { set_err(err, errcap, "unknown curve %u or null scalar", curve); return SSO_E_ARG; }
-  Ctx c(err, errcap);
-  int rc = c.init(device);
-  if (rc) return rc;
-  uint32_t* d_status;
-  if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
-  if (group > 1) { set_err(err, errcap, "unknown group %u", group); return SSO_E_ARG; }
-  // vectors longer than the span of one tau table (2^24 indices) are processed in segments, each with its own table base
-  CurveSizes cs;
-  curve_sizes(curve, cs);
-  const uint64_t in_sz = point_size(cs, group, in_compressed), out_sz = point_size(cs, group, out_compressed);
-  const uint64_t SEG = 1ull << 22;
-  for (uint64_t off = 0; off < n; off += SEG) {
-    uint64_t m = n - off < SEG ? n - off : SEG;
-    if ((rc = single_vector(c, ops, group, (const uint8_t*)d_in + off * in_sz, in_compressed, m, first_index + off, tau, coeff, 0,
-                            (uint8_t*)d_out + off * out_sz, out_compressed, check_input, d_status, err, errcap))) return rc;
-  }
-  if ((rc = sync_all(c, err, errcap))) return rc;
-  return check_status(c, d_status, "batch_exp input", err, errcap);
+  return batch_scalar_dev(curve, group, d_in, in_compressed, n, first_index, tau, coeff, 0, d_out, out_compressed, check_input, device, err, errcap);
 }
 
 int32_t sso_batch_mul_dev(uint32_t curve, uint32_t group, const void* d_in, uint32_t in_compressed, uint64_t n,
                           const uint8_t* scalar, void* d_out, uint32_t out_compressed, uint32_t check_input,
                           int device, char* err, size_t errcap) {
-  const CurveOps* ops = ops_for(curve);
-  if (!ops || !scalar) { set_err(err, errcap, "unknown curve %u or null scalar", curve); return SSO_E_ARG; }
-  Ctx c(err, errcap);
-  int rc = c.init(device);
-  if (rc) return rc;
-  uint32_t* d_status;
-  if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
-  if (group > 1) { set_err(err, errcap, "unknown group %u", group); return SSO_E_ARG; }
-  std::vector<uint8_t> one(ops->fr_bytes, 0);
-  one[0] = 1;
-  // vectors longer than the table span are processed in segments (the scalar is index-independent)
-  CurveSizes cs;
-  curve_sizes(curve, cs);
-  uint64_t in_sz = group == GROUP_G1 ? (in_compressed ? cs.g1c : cs.g1u) : (in_compressed ? cs.g2c : cs.g2u);
-  uint64_t out_sz = group == GROUP_G1 ? (out_compressed ? cs.g1c : cs.g1u) : (out_compressed ? cs.g2c : cs.g2u);
-  const uint64_t SEG = 1ull << 22;
-  for (uint64_t off = 0; off < n; off += SEG) {
-    uint64_t m = n - off < SEG ? n - off : SEG;
-    if ((rc = single_vector(c, ops, group, (const uint8_t*)d_in + off * in_sz, in_compressed, m, 0, one.data(), scalar, 1,
-                            (uint8_t*)d_out + off * out_sz, out_compressed, check_input, d_status, err, errcap))) return rc;
-  }
-  if ((rc = sync_all(c, err, errcap))) return rc;
-  return check_status(c, d_status, "batch_mul input", err, errcap);
+  return batch_scalar_dev(curve, group, d_in, in_compressed, n, 0, nullptr, scalar, 1, d_out, out_compressed, check_input, device, err, errcap);
 }
 
 int32_t sso_reencode_dev(uint32_t curve, uint32_t group, const void* d_in, uint32_t in_compressed, uint64_t n,
@@ -295,7 +299,7 @@ int32_t sso_reencode_dev(uint32_t curve, uint32_t group, const void* d_in, uint3
   int rc = c.init(device);
   if (rc) return rc;
   uint32_t* d_status;
-  if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
+  if ((rc = status_buffer(c, &d_status, 0, true, err, errcap))) return rc;
   if ((rc = ops->reencode(c, 0, group, (const uint8_t*)d_in, in_compressed, n, (uint8_t*)d_out, out_compressed, check,
                           subgroup_check, nullptr, d_status, err, errcap))) return rc;
   if ((rc = sync_all(c, err, errcap))) return rc;
@@ -311,22 +315,15 @@ int32_t sso_power_pairs_dev(uint32_t curve, uint32_t group, const void* d_in, ui
   if (n < 2) { set_err(err, errcap, "power_pairs needs at least two elements"); return SSO_E_ARG; }
   CurveSizes cs;
   curve_sizes(curve, cs);
-  uint64_t usz = group == GROUP_G1 ? cs.g1u : cs.g2u;
+  const size_t usz = point_size(cs, group, 0);
   if (out_len != 2 * usz) { set_err(err, errcap, "output buffer must hold two uncompressed points (%llu bytes)", (unsigned long long)(2 * usz)); return SSO_E_ARG; }
   Ctx c(err, errcap);
   int rc = c.init(device);
   if (rc) return rc;
-  uint32_t *d_status, *d_aff;
-  uint8_t* d_out;
-  if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
-  if ((rc = c.alloc((void**)&d_aff, n * ops->aff_words[group] * 4))) return rc;
-  if ((rc = c.alloc((void**)&d_out, 2 * usz))) return rc;
-  if ((rc = ops->reencode(c, 0, group, (const uint8_t*)d_in, in_compressed, n, nullptr, 0, check, subgroup_check, d_aff, d_status, err, errcap))) return rc;
-  if ((rc = ops->msm_pairs(c, 0, group, d_aff, d_aff + ops->aff_words[group], n - 1, seed32, nullptr, d_out, err, errcap))) return rc;
-  if ((rc = sync_all(c, err, errcap))) return rc;
-  if ((rc = check_status(c, d_status, "point", err, errcap))) return rc;
-  CUDA_TRY(cudaMemcpy(out_pair, d_out, 2 * usz, cudaMemcpyDeviceToHost));
-  return SSO_OK;
+  uint32_t* d_status;
+  if ((rc = status_buffer(c, &d_status, 0, true, err, errcap))) return rc;
+  return pair_to_host(c, ops, group, usz, n, {(const uint8_t*)d_in, in_compressed, check, subgroup_check}, {}, seed32, nullptr, d_status,
+                      "point", out_pair, err, errcap);
 }
 
 // K3 + K5: (sum r_i a_i, sum r_i b_i) [merge_pairs] for two vectors of n points each
@@ -338,24 +335,15 @@ int32_t sso_merge_pairs_dev(uint32_t curve, uint32_t group, const void* d_a, con
   if (n < 1) { set_err(err, errcap, "merge_pairs needs at least one element"); return SSO_E_ARG; }
   CurveSizes cs;
   curve_sizes(curve, cs);
-  uint64_t usz = group == GROUP_G1 ? cs.g1u : cs.g2u;
+  const size_t usz = point_size(cs, group, 0);
   if (out_len != 2 * usz) { set_err(err, errcap, "output buffer must hold two uncompressed points (%llu bytes)", (unsigned long long)(2 * usz)); return SSO_E_ARG; }
   Ctx c(err, errcap);
   int rc = c.init(device);
   if (rc) return rc;
-  uint32_t *d_status, *d_aff_a, *d_aff_b;
-  uint8_t* d_out;
-  if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
-  if ((rc = c.alloc((void**)&d_aff_a, n * ops->aff_words[group] * 4))) return rc;
-  if ((rc = c.alloc((void**)&d_aff_b, n * ops->aff_words[group] * 4))) return rc;
-  if ((rc = c.alloc((void**)&d_out, 2 * usz))) return rc;
-  if ((rc = ops->reencode(c, 0, group, (const uint8_t*)d_a, in_compressed, n, nullptr, 0, check, subgroup_check, d_aff_a, d_status, err, errcap))) return rc;
-  if ((rc = ops->reencode(c, 0, group, (const uint8_t*)d_b, in_compressed, n, nullptr, 0, check, subgroup_check, d_aff_b, d_status, err, errcap))) return rc;
-  if ((rc = ops->msm_pairs(c, 0, group, d_aff_a, d_aff_b, n, seed32, nullptr, d_out, err, errcap))) return rc;
-  if ((rc = sync_all(c, err, errcap))) return rc;
-  if ((rc = check_status(c, d_status, "point", err, errcap))) return rc;
-  CUDA_TRY(cudaMemcpy(out_pair, d_out, 2 * usz, cudaMemcpyDeviceToHost));
-  return SSO_OK;
+  uint32_t* d_status;
+  if ((rc = status_buffer(c, &d_status, 0, true, err, errcap))) return rc;
+  return pair_to_host(c, ops, group, usz, n, {(const uint8_t*)d_a, in_compressed, check, subgroup_check},
+                      {(const uint8_t*)d_b, in_compressed, check, subgroup_check}, seed32, nullptr, d_status, "point", out_pair, err, errcap);
 }
 
 // K8: batch of same_ratio checks on host buffers
@@ -394,7 +382,7 @@ int32_t sso_p1_contribute_dev(const sso_p1_params_t* p, const void* d_challenge,
   Ctx c(err, errcap);
   if ((rc = c.init(device, 2))) return rc;
   uint32_t* d_status;
-  if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
+  if ((rc = status_buffer(c, &d_status, 0, true, err, errcap))) return rc;
   if ((rc = p1_contribute_streams(c, ops, L, (const uint8_t*)d_challenge, (uint8_t*)d_response, tau, alpha, beta, check_input, d_status, err, errcap))) return rc;
   if ((rc = sync_all(c, err, errcap))) return rc;
   return check_status(c, d_status, "challenge", err, errcap);
@@ -418,7 +406,7 @@ static int32_t contribute_streamed(const sso_p1_params_t* p, const P1Layout& L, 
   Participants P;
   if ((rc = resolve_participants(nullptr, 0, device, p->contribution_mode == SSO_MODE_FULL, P, err, errcap))) return rc;
   std::thread hasher([=] { blake2b_512(challenge, L.acc_size, response); });
-  struct Joiner { std::thread& t; ~Joiner() { if (t.joinable()) t.join(); } } joiner{hasher};
+  JoinOnExit join_hasher{hasher};
   Ctx c(err, errcap);
   if ((rc = c.init(P.devices[0], 1))) return rc;
   std::vector<uint8_t> scalars;
@@ -460,7 +448,7 @@ static int32_t contribute_buf_core(const sso_p1_params_t* p, const uint8_t* chal
   // the hash-chain link is computed on the host while the GPU works; with a seed it starts before the key generation
   // (whose first stage is a ~19 ms single-thread kernel the host would otherwise wait for)
   std::thread hasher;
-  struct Joiner { std::thread& t; ~Joiner() { if (t.joinable()) t.join(); } } joiner{hasher};
+  JoinOnExit join_hasher{hasher};
   if (seed32) {
     hasher = std::thread([=] { blake2b_512(challenge, challenge_len, response); });
     scalars.resize(3 * (size_t)L.cs.fr);
@@ -474,7 +462,7 @@ static int32_t contribute_buf_core(const sso_p1_params_t* p, const uint8_t* chal
   uint32_t* d_status;
   if ((rc = c.alloc((void**)&d_ch, L.acc_size))) return rc;
   if ((rc = c.alloc((void**)&d_resp, L.contrib_size))) return rc;
-  if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
+  if ((rc = status_buffer(c, &d_status, 0, true, err, errcap))) return rc;
   c.mark("scratch allocated");
   // stream-ordered: the kernels below are enqueued behind the copy, and the host goes straight on to hashing
   CUDA_TRY(cudaMemcpyAsync(d_ch, challenge, L.acc_size, cudaMemcpyHostToDevice, c.s[0]));
@@ -655,14 +643,14 @@ int32_t sso_points_sum(uint32_t curve, uint32_t group, const uint8_t* points, ui
   const CurveOps* ops = ops_for(curve);
   CurveSizes cs;
   if (!ops || group > 1 || !curve_sizes(curve, cs)) { set_err(err, errcap, "unknown curve/group %u/%u", curve, group); return SSO_E_ARG; }
-  uint64_t usz = group == GROUP_G1 ? cs.g1u : cs.g2u;
+  const size_t usz = point_size(cs, group, 0);
   if (out_len != usz || n == 0 || n > 65536) { set_err(err, errcap, "points_sum: bad sizes"); return SSO_E_ARG; }
   Ctx c(err, errcap);
   int rc = c.init(device);
   if (rc) return rc;
   uint8_t *d_in, *d_out;
   uint32_t* d_status;
-  if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
+  if ((rc = status_buffer(c, &d_status, 0, true, err, errcap))) return rc;
   if ((rc = c.alloc((void**)&d_in, n * usz))) return rc;
   if ((rc = c.alloc((void**)&d_out, usz))) return rc;
   CUDA_TRY(cudaMemcpyAsync(d_in, points, n * usz, cudaMemcpyHostToDevice, c.s[0]));
@@ -679,7 +667,7 @@ int32_t sso_p2_scale_queries_buf(uint32_t curve, const uint8_t* in, size_t in_le
                                  int device, char* err, size_t errcap) {
   CurveSizes cs;
   if (!curve_sizes(curve, cs) || !in || !out || !delta_inv) { set_err(err, errcap, "unknown curve %u or null argument", curve); return SSO_E_ARG; }
-  size_t isz = in_compressed ? cs.g1c : cs.g1u, osz = out_compressed ? cs.g1c : cs.g1u;
+  const size_t isz = point_size(cs, GROUP_G1, in_compressed), osz = point_size(cs, GROUP_G1, out_compressed);
   if (in_len != n * isz || out_len != n * osz) { set_err(err, errcap, "query buffers have the wrong size for %llu points", (unsigned long long)n); return SSO_E_ARG; }
   if (n == 0) return SSO_OK;
   Ctx c(err, errcap);
@@ -703,29 +691,22 @@ int32_t sso_p2_verify_queries_buf(uint32_t curve, const uint8_t* before, size_t 
   const CurveOps* ops = ops_for(curve);
   CurveSizes cs;
   if (!ops || !curve_sizes(curve, cs) || !before || !after || !delta_g2_before || !delta_g2_after) { set_err(err, errcap, "unknown curve %u or null argument", curve); return SSO_E_ARG; }
-  size_t bsz = before_compressed ? cs.g1c : cs.g1u, asz = after_compressed ? cs.g1c : cs.g1u;
+  const size_t bsz = point_size(cs, GROUP_G1, before_compressed), asz = point_size(cs, GROUP_G1, after_compressed);
   if (before_len != n * bsz || after_len != n * asz || n == 0) { set_err(err, errcap, "query buffers have the wrong size for %llu points", (unsigned long long)n); return SSO_E_ARG; }
   Ctx c(err, errcap);
   int rc = c.init(device);
   if (rc) return rc;
-  uint8_t *d_b, *d_a, *d_pair;
-  uint32_t *d_status, *d_aff_b, *d_aff_a;
-  if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
+  uint8_t *d_b, *d_a;
+  uint32_t* d_status;
+  if ((rc = status_buffer(c, &d_status, 0, true, err, errcap))) return rc;
   if ((rc = c.alloc((void**)&d_b, before_len))) return rc;
   if ((rc = c.alloc((void**)&d_a, after_len))) return rc;
-  if ((rc = c.alloc((void**)&d_aff_b, n * ops->aff_words[0] * 4))) return rc;
-  if ((rc = c.alloc((void**)&d_aff_a, n * ops->aff_words[0] * 4))) return rc;
-  if ((rc = c.alloc((void**)&d_pair, 2 * cs.g1u))) return rc;
   CUDA_TRY(cudaMemcpyAsync(d_b, before, before_len, cudaMemcpyHostToDevice, c.s[0]));
   CUDA_TRY(cudaMemcpyAsync(d_a, after, after_len, cudaMemcpyHostToDevice, c.s[0]));
-  if ((rc = ops->reencode(c, 0, GROUP_G1, d_b, before_compressed, n, nullptr, 0, SSO_CHECK_NO, 0, d_aff_b, d_status, err, errcap))) return rc;
-  if ((rc = ops->reencode(c, 0, GROUP_G1, d_a, after_compressed, n, nullptr, 0, check, subgroup_check, d_aff_a, d_status, err, errcap))) return rc;
   const uint64_t tweak[4] = {TWEAK_P2_VERIFY, n, 0, 0};
-  if ((rc = ops->msm_pairs(c, 0, GROUP_G1, d_aff_b, d_aff_a, n, rlc_seed32, tweak, d_pair, err, errcap))) return rc;
-  if ((rc = sync_all(c, err, errcap))) return rc;
-  if ((rc = check_status(c, d_status, "query", err, errcap))) return rc == SSO_E_INPUT ? SSO_E_VERIFY : rc;
   std::vector<uint8_t> pair(2 * cs.g1u);
-  CUDA_TRY(cudaMemcpy(pair.data(), d_pair, pair.size(), cudaMemcpyDeviceToHost));
+  if ((rc = pair_to_host(c, ops, GROUP_G1, cs.g1u, n, {d_b, before_compressed, SSO_CHECK_NO, 0}, {d_a, after_compressed, check, subgroup_check},
+                         rlc_seed32, tweak, d_status, "query", pair.data(), err, errcap))) return rc == SSO_E_INPUT ? SSO_E_VERIFY : rc;
   std::vector<RatioCheck> checks;
   add_check(checks, "phase-2 query vs delta_g2", pair.data(), pair.data() + cs.g1u, cs.g1u, delta_g2_after, delta_g2_before, cs.g2u);
   return run_checks(c, ops, checks, err, errcap);
@@ -825,7 +806,7 @@ int32_t sso_p1_set_generators(uint32_t curve, const uint8_t* g1_uncompressed, si
   uint8_t* d_pts;
   uint32_t* d_status;
   if ((rc = c.alloc((void**)&d_pts, cs.g1u + cs.g2u))) return rc;
-  if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
+  if ((rc = status_buffer(c, &d_status, 0, true, err, errcap))) return rc;
   CUDA_TRY(cudaMemcpyAsync(d_pts, g1_uncompressed, cs.g1u, cudaMemcpyHostToDevice, c.s[0]));
   CUDA_TRY(cudaMemcpyAsync(d_pts + cs.g1u, g2_uncompressed, cs.g2u, cudaMemcpyHostToDevice, c.s[0]));
   if ((rc = ops->reencode(c, 0, GROUP_G1, d_pts, 0, 1, nullptr, 0, CHECK_FULL, 1, nullptr, d_status, err, errcap))) return rc;
@@ -866,10 +847,9 @@ int fill_generators(Ctx& c, int si, const CurveOps* ops, const CurveSizes& cs, u
   uint32_t* d_status;
   if ((rc = c.alloc((void**)&d_u, usz, si))) return rc;
   if ((rc = c.alloc((void**)&d_pat, osz, si))) return rc;
-  if ((rc = c.alloc((void**)&d_status, STATUS_BYTES, si))) return rc;
+  if ((rc = status_buffer(c, &d_status, si, false, err, errcap))) return rc;
   c.staging.emplace_back((usz + 3) / 4, 0u);
   memcpy(c.staging.back().data(), pt.data(), usz);
-  CUDA_TRY(cudaMemsetAsync(d_status, 0, STATUS_BYTES, c.s[si]));
   CUDA_TRY(cudaMemcpyAsync(d_u, c.staging.back().data(), usz, cudaMemcpyHostToDevice, c.s[si]));
   if ((rc = ops->reencode(c, si, group, d_u, 0, 1, d_pat, out_compressed, CHECK_NO, 0, nullptr, d_status, err, errcap))) return rc;
   uint64_t total = n * osz;
@@ -882,6 +862,28 @@ int fill_generators(Ctx& c, int si, const CurveOps* ops, const CurveSizes& cs, u
 }
 
 bool is_coop(const sso_p1_params_t* p) { return p && p->contribution_mode == SSO_MODE_FULL && dist_state().on; }
+
+// A file call with one mapped output of `out_size` bytes, made by every rank of the process group when `coop` (each computes
+// its pieces into the shared mapping), else by this process alone.  The ranks agree after every step, so that a rank that
+// failed makes the others return instead of waiting in a collective:
+//   1. inputs() — every rank; then the lead rank creates the partial output
+//   2. the other ranks map that partial output; then work(out) — every rank
+//   3. the lead rank writes its small outputs with finish(outputs, out); every rank commits (the others only detach)
+template <class Inputs, class Work, class Finish>
+int32_t file_call(bool coop, const char* out_fn, size_t out_size, Inputs inputs, Work work, Finish finish, char* err, size_t errcap) {
+  const bool lead = !coop || dist_state().rank == 0;
+  Outputs outs;
+  uint8_t* out = nullptr;
+  int32_t rc = inputs();
+  if (!rc && lead) rc = outs.create_mapped(out_fn, out_size, true, &out, err, errcap);
+  if ((rc = coop_result(coop, rc, err, errcap))) return rc;
+  if (!lead) rc = outs.create_mapped(out_fn, out_size, false, &out, err, errcap);
+  if (!rc) rc = work(out);
+  if ((rc = coop_result(coop, rc, err, errcap))) return rc;
+  if (lead) rc = finish(outs, out);
+  if (!rc) rc = outs.commit(err, errcap);
+  return coop_result(coop, rc, err, errcap);
+}
 }  // namespace
 
 extern "C" {
@@ -896,9 +898,10 @@ int32_t sso_p1_new_challenge_file(const char* challenge_fn, const char* challeng
   if (rc) return rc;
   if (!challenge_fn || !challenge_hash_fn) { set_err(err, errcap, "null argument"); return SSO_E_ARG; }
   const CurveOps* ops = ops_for(p->curve);
-  MappedFile out;
-  if ((rc = out.create(challenge_fn, L.acc_size, true, err, errcap))) return rc;
-  blake2b_512(nullptr, 0, out.p);
+  Outputs outs;
+  uint8_t* out;
+  if ((rc = outs.create_mapped(challenge_fn, L.acc_size, true, &out, err, errcap))) return rc;
+  blake2b_512(nullptr, 0, out);
   const uint64_t counts[5] = {L.g1n, L.on, L.on, L.on, 1};
   static const uint32_t groups[5] = {GROUP_G1, GROUP_G2, GROUP_G1, GROUP_G1, GROUP_G2};
   {
@@ -912,17 +915,13 @@ int32_t sso_p1_new_challenge_file(const char* challenge_fn, const char* challeng
         uint8_t* d_buf;
         if ((rc = c.alloc((void**)&d_buf, cnt * usz))) return rc;
         if ((rc = fill_generators(c, 0, ops, L.cs, p->curve, groups[v], cnt, d_buf, 0, err, errcap))) return rc;
-        CUDA_TRY(cudaMemcpyAsync(out.p + L.off_u[v] + lo * usz, d_buf, cnt * usz, cudaMemcpyDeviceToHost, c.s[0]));
+        CUDA_TRY(cudaMemcpyAsync(out + L.off_u[v] + lo * usz, d_buf, cnt * usz, cudaMemcpyDeviceToHost, c.s[0]));
         if ((rc = c.recycle())) return rc;
       }
     }
   }
-  uint8_t h[64];
-  blake2b_512(out.p, L.acc_size, h);
-  std::vector<SmallFile> small;
-  if ((rc = write_small(small, challenge_hash_fn, h, 64, err, errcap))) return rc;
-  if ((rc = out.commit(err, errcap))) { discard_small(small); return rc; }
-  return commit_small(small, err, errcap);
+  if ((rc = outs.write_hash(challenge_hash_fn, out, L.acc_size, err, errcap))) return rc;
+  return outs.commit(err, errcap);
 }
 
 // phase1_cli::contribute(challenge_fn, challenge_hash_fn, response_fn, response_hash_fn, check_input, batch_exp_mode, params, rng)
@@ -936,54 +935,35 @@ int32_t sso_p1_contribute_file(const sso_p1_params_t* p, const char* challenge_f
   int rc = p1_layout(p, L, err, errcap);
   if (rc) return rc;
   if (!challenge_fn || !challenge_hash_fn || !response_fn || !response_hash_fn || !seed32) { set_err(err, errcap, "null argument"); return SSO_E_ARG; }
-  const bool coop = is_coop(p), lead = !coop || dist_state().rank == 0;
   if (!needs_streaming(p, L)) {
     // chunk-sized call: page-locked staging in and out (files.cuh), outputs written whole and renamed
     PinnedLease in(L.acc_size), out(L.contrib_size);
     if (!in.b.p || !out.b.p) { set_err(err, errcap, "cannot allocate page-locked staging buffers"); return SSO_E_CUDA; }
-    struct stat st;
-    if (stat(response_fn, &st) == 0) { set_err(err, errcap, "cannot create %s (outputs must not exist)", response_fn); return SSO_E_IO; }
+    if ((rc = refuse_existing(response_fn, err, errcap))) return rc;
     if ((rc = read_file_into(challenge_fn, in.b.p, L.acc_size, err, errcap))) return rc;
     if ((rc = contribute_buf_core(p, in.b.p, L.acc_size, out.b.p, L.contrib_size, nullptr, nullptr, nullptr, nullptr, 0, seed32, check_input, device, err, errcap))) return rc;
-    uint8_t h[64];
-    blake2b_512(out.b.p, L.contrib_size, h);
-    std::vector<SmallFile> small;
-    if ((rc = write_small(small, response_fn, out.b.p, L.contrib_size, err, errcap))) return rc;
-    if ((rc = write_small(small, challenge_hash_fn, out.b.p, 64, err, errcap))) { discard_small(small); return rc; }     // response[0..64) = hash(challenge)
-    if ((rc = write_small(small, response_hash_fn, h, 64, err, errcap))) { discard_small(small); return rc; }
-    return commit_small(small, err, errcap);
+    Outputs outs;
+    if ((rc = outs.write_whole(response_fn, out.b.p, L.contrib_size, err, errcap))) return rc;
+    if ((rc = outs.write_whole(challenge_hash_fn, out.b.p, 64, err, errcap))) return rc;     // response[0..64) = hash(challenge)
+    if ((rc = outs.write_hash(response_hash_fn, out.b.p, L.contrib_size, err, errcap))) return rc;
+    return outs.commit(err, errcap);
   }
-  MappedFile in, out;
-  std::vector<SmallFile> small;
-  auto body = [&]() -> int32_t {
-    int32_t rc;
-    if ((rc = in.open_ro(challenge_fn, err, errcap))) return rc;
-    if (in.len != L.acc_size) { set_err(err, errcap, "The size of challenge file should be correct: %zu != %llu", in.len, (unsigned long long)L.acc_size); return SSO_E_ARG; }
-    if (lead && (rc = out.create(response_fn, L.contrib_size, true, err, errcap))) return rc;
-    return SSO_OK;
-  };
-  rc = coop_result(coop, body(), err, errcap);                       // the leader's partial file exists before the others open it
-  if (rc) return rc;
-  auto body2 = [&]() -> int32_t {
-    int32_t rc;
-    if (!lead && (rc = out.create(response_fn, L.contrib_size, false, err, errcap))) return rc;
-    return contribute_buf_core(p, in.p, in.len, out.p, out.len, nullptr, nullptr, nullptr, nullptr, 0, seed32, check_input, device, err, errcap);
-  };
-  rc = coop_result(coop, body2(), err, errcap);                      // every rank's pieces are in the shared mapping
-  if (rc) return rc;
-  auto body3 = [&]() -> int32_t {
-    int32_t rc;
-    if (!lead) { out.unmap(); out.committed = true; return SSO_OK; }
-    uint8_t h[64];
-    if ((rc = write_small(small, challenge_hash_fn, out.p, 64, err, errcap))) return rc;       // response[0..64) = hash(challenge)
-    blake2b_512(out.p, out.len, h);
-    if ((rc = write_small(small, response_hash_fn, h, 64, err, errcap))) return rc;
-    if ((rc = out.commit(err, errcap))) return rc;
-    return commit_small(small, err, errcap);
-  };
-  rc = body3();
-  if (rc) discard_small(small);
-  return coop_result(coop, rc, err, errcap);
+  MappedFile in;
+  return file_call(is_coop(p), response_fn, L.contrib_size,
+      [&]() -> int32_t {
+        int32_t rc;
+        if ((rc = in.open_ro(challenge_fn, err, errcap))) return rc;
+        if (in.len != L.acc_size) { set_err(err, errcap, "The size of challenge file should be correct: %zu != %llu", in.len, (unsigned long long)L.acc_size); return SSO_E_ARG; }
+        return SSO_OK;
+      },
+      [&](uint8_t* out) {
+        return contribute_buf_core(p, in.p, in.len, out, L.contrib_size, nullptr, nullptr, nullptr, nullptr, 0, seed32, check_input, device, err, errcap);
+      },
+      [&](Outputs& outs, const uint8_t* out) {
+        int32_t rc;
+        if ((rc = outs.write_whole(challenge_hash_fn, out, 64, err, errcap))) return rc;        // response[0..64) = hash(challenge)
+        return outs.write_hash(response_hash_fn, out, L.contrib_size, err, errcap);
+      }, err, errcap);
 }
 
 // phase1_cli::transform_pok_and_correctness(challenge_fn, challenge_hash_fn, check_input, response_fn, response_hash_fn,
@@ -997,61 +977,43 @@ int32_t sso_p1_verify_chunk_file(const sso_p1_params_t* p, const char* challenge
   int rc = p1_layout(p, L, err, errcap);
   if (rc) return rc;
   if (!challenge_fn || !challenge_hash_fn || !response_fn || !response_hash_fn || !new_challenge_fn || !new_challenge_hash_fn) { set_err(err, errcap, "null argument"); return SSO_E_ARG; }
-  const bool coop = is_coop(p), lead = !coop || dist_state().rank == 0;
   if (!needs_streaming(p, L)) {
     PinnedLease chb(L.acc_size), respb(L.contrib_size), outb(L.acc_size);
     if (!chb.b.p || !respb.b.p || !outb.b.p) { set_err(err, errcap, "cannot allocate page-locked staging buffers"); return SSO_E_CUDA; }
-    struct stat st;
-    if (stat(new_challenge_fn, &st) == 0) { set_err(err, errcap, "cannot create %s (outputs must not exist)", new_challenge_fn); return SSO_E_IO; }
+    if ((rc = refuse_existing(new_challenge_fn, err, errcap))) return rc;
     if ((rc = read_file_into(challenge_fn, chb.b.p, L.acc_size, err, errcap))) return rc;
     if ((rc = read_file_into(response_fn, respb.b.p, L.contrib_size, err, errcap))) return rc;
-    uint8_t ch_hash[64], h[64];
+    uint8_t ch_hash[64];
     if ((rc = verify_chunk_core(p, chb.b.p, L.acc_size, respb.b.p, L.contrib_size, outb.b.p, L.acc_size, check_input, check_output, subgroup_check_mode,
                                 ratio_check, nullptr, device, ch_hash, err, errcap))) return rc;
-    blake2b_512(outb.b.p, L.acc_size, h);
-    std::vector<SmallFile> small;
-    if ((rc = write_small(small, new_challenge_fn, outb.b.p, L.acc_size, err, errcap))) return rc;
-    if ((rc = write_small(small, challenge_hash_fn, ch_hash, 64, err, errcap))) { discard_small(small); return rc; }
-    if ((rc = write_small(small, response_hash_fn, outb.b.p, 64, err, errcap))) { discard_small(small); return rc; }        // new_challenge[0..64) = hash(response)
-    if ((rc = write_small(small, new_challenge_hash_fn, h, 64, err, errcap))) { discard_small(small); return rc; }
-    return commit_small(small, err, errcap);
+    Outputs outs;
+    if ((rc = outs.write_whole(new_challenge_fn, outb.b.p, L.acc_size, err, errcap))) return rc;
+    if ((rc = outs.write_whole(challenge_hash_fn, ch_hash, 64, err, errcap))) return rc;
+    if ((rc = outs.write_whole(response_hash_fn, outb.b.p, 64, err, errcap))) return rc;        // new_challenge[0..64) = hash(response)
+    if ((rc = outs.write_hash(new_challenge_hash_fn, outb.b.p, L.acc_size, err, errcap))) return rc;
+    return outs.commit(err, errcap);
   }
-  MappedFile ch, resp, out;
-  std::vector<SmallFile> small;
+  MappedFile ch, resp;
   uint8_t ch_hash[64];
-  auto body = [&]() -> int32_t {
-    int32_t rc;
-    if ((rc = ch.open_ro(challenge_fn, err, errcap))) return rc;
-    if ((rc = resp.open_ro(response_fn, err, errcap))) return rc;
-    if (ch.len != L.acc_size) { set_err(err, errcap, "The size of challenge file should be correct: %zu != %llu", ch.len, (unsigned long long)L.acc_size); return SSO_E_ARG; }
-    if (resp.len != L.contrib_size) { set_err(err, errcap, "The size of response file should be correct: %zu != %llu", resp.len, (unsigned long long)L.contrib_size); return SSO_E_ARG; }
-    if (lead && (rc = out.create(new_challenge_fn, L.acc_size, true, err, errcap))) return rc;
-    return SSO_OK;
-  };
-  rc = coop_result(coop, body(), err, errcap);
-  if (rc) return rc;
-  auto body2 = [&]() -> int32_t {
-    int32_t rc;
-    if (!lead && (rc = out.create(new_challenge_fn, L.acc_size, false, err, errcap))) return rc;
-    return verify_chunk_core(p, ch.p, ch.len, resp.p, resp.len, out.p, out.len, check_input, check_output, subgroup_check_mode, ratio_check,
-                             nullptr, device, ch_hash, err, errcap);
-  };
-  rc = coop_result(coop, body2(), err, errcap);
-  if (rc) return rc;
-  auto body3 = [&]() -> int32_t {
-    int32_t rc;
-    if (!lead) { out.unmap(); out.committed = true; return SSO_OK; }
-    uint8_t h[64];
-    if ((rc = write_small(small, challenge_hash_fn, ch_hash, 64, err, errcap))) return rc;
-    if ((rc = write_small(small, response_hash_fn, out.p, 64, err, errcap))) return rc;         // new_challenge[0..64) = hash(response)
-    blake2b_512(out.p, out.len, h);
-    if ((rc = write_small(small, new_challenge_hash_fn, h, 64, err, errcap))) return rc;
-    if ((rc = out.commit(err, errcap))) return rc;
-    return commit_small(small, err, errcap);
-  };
-  rc = body3();
-  if (rc) discard_small(small);
-  return coop_result(coop, rc, err, errcap);
+  return file_call(is_coop(p), new_challenge_fn, L.acc_size,
+      [&]() -> int32_t {
+        int32_t rc;
+        if ((rc = ch.open_ro(challenge_fn, err, errcap))) return rc;
+        if ((rc = resp.open_ro(response_fn, err, errcap))) return rc;
+        if (ch.len != L.acc_size) { set_err(err, errcap, "The size of challenge file should be correct: %zu != %llu", ch.len, (unsigned long long)L.acc_size); return SSO_E_ARG; }
+        if (resp.len != L.contrib_size) { set_err(err, errcap, "The size of response file should be correct: %zu != %llu", resp.len, (unsigned long long)L.contrib_size); return SSO_E_ARG; }
+        return SSO_OK;
+      },
+      [&](uint8_t* out) {
+        return verify_chunk_core(p, ch.p, ch.len, resp.p, resp.len, out, L.acc_size, check_input, check_output, subgroup_check_mode, ratio_check,
+                                 nullptr, device, ch_hash, err, errcap);
+      },
+      [&](Outputs& outs, const uint8_t* out) {
+        int32_t rc;
+        if ((rc = outs.write_whole(challenge_hash_fn, ch_hash, 64, err, errcap))) return rc;
+        if ((rc = outs.write_whole(response_hash_fn, out, 64, err, errcap))) return rc;         // new_challenge[0..64) = hash(response)
+        return outs.write_hash(new_challenge_hash_fn, out, L.acc_size, err, errcap);
+      }, err, errcap);
 }
 
 // phase1_cli::combine(response_list_fn, combined_fn, params) — reference src/bin/verify_transcript.rs:603-607,
@@ -1069,59 +1031,49 @@ int32_t sso_p1_combine_file(const char* response_list_fn, const char* combined_f
   if (rc) return rc;
   if (p->chunk_size == 0) { set_err(err, errcap, "combine needs the chunk size of the ceremony"); return SSO_E_ARG; }
   const CurveOps* ops = ops_for(p->curve);
-  const bool coop = dist_state().on, lead = !coop || dist_state().rank == 0;
   // the list of response files
   std::vector<std::string> names;
   {
-    std::vector<uint8_t> txt;
-    if ((rc = read_file(response_list_fn, txt, err, errcap))) return rc;
+    MappedFile txt;
+    if ((rc = txt.open_ro(response_list_fn, err, errcap))) return rc;
     std::string cur;
-    for (uint8_t ch : txt) {
+    for (size_t i = 0; i < txt.len; i++) {
+      const char ch = (char)txt.p[i];
       if (ch == '\n' || ch == '\r') { if (!cur.empty()) names.push_back(cur); cur.clear(); }
-      else cur.push_back((char)ch);
+      else cur.push_back(ch);
     }
     if (!cur.empty()) names.push_back(cur);
   }
   const uint64_t nchunks = (LF.powers_g1_length + p->chunk_size - 1) / p->chunk_size;
   if (names.size() != nchunks) { set_err(err, errcap, "response list names %zu files, the ceremony has %llu chunks", names.size(), (unsigned long long)nchunks); return SSO_E_ARG; }
   std::vector<std::unique_ptr<MappedFile>> ins(nchunks);
-  MappedFile out;
-  std::vector<RVec> vecs;
   static const uint32_t groups[5] = {GROUP_G1, GROUP_G2, GROUP_G1, GROUP_G1, GROUP_G2};
   static const char* vnames[5] = {"tau_g1", "tau_g2", "alpha_g1", "beta_g1", "beta_g2"};
-  auto body = [&]() -> int32_t {
-    int32_t rc;
-    if (lead && (rc = out.create(combined_fn, LF.acc_size, true, err, errcap))) return rc;
-    return SSO_OK;
-  };
-  if ((rc = coop_result(coop, body(), err, errcap))) return rc;
-  auto body2 = [&]() -> int32_t {
-    int32_t rc;
-    if (!lead && (rc = out.create(combined_fn, LF.acc_size, false, err, errcap))) return rc;
-    for (uint64_t k = 0; k < nchunks; k++) {
-      sso_p1_params_t pk = *p;
-      pk.contribution_mode = SSO_MODE_CHUNKED; pk.chunk_index = k;
-      P1Layout L;
-      if ((rc = p1_layout(&pk, L, err, errcap))) return rc;
-      ins[k].reset(new MappedFile());
-      if ((rc = ins[k]->open_ro(names[k].c_str(), err, errcap))) return rc;
-      if (ins[k]->len != L.contrib_size) { set_err(err, errcap, "The size of response file %s should be correct: %zu != %llu", names[k].c_str(), ins[k]->len, (unsigned long long)L.contrib_size); return SSO_E_ARG; }
-      const uint64_t counts[5] = {L.g1n, L.on, L.on, L.on, k == 0 ? 1ull : 0ull};       // beta_g2 is taken from the first chunk
-      for (int v = 0; v < 5; v++) {
-        if (counts[v] == 0) continue;
-        const size_t usz = point_size(L.cs, groups[v], 0);
-        vecs.push_back({groups[v], ins[k]->p + L.off_c[v], 1, counts[v], out.p + LF.off_u[v] + (v == 4 ? 0 : L.start * usz), 0, 0,
-                        CHECK_NO, 0, 0, vnames[v]});
-      }
-    }
-    Participants P;
-    if ((rc = resolve_participants(devices, ndev, device, true, P, err, errcap))) return rc;
-    return stream_reencode(ops, LF.cs, vecs, p->batch_size, nullptr, 0, P, nullptr, err, errcap);
-  };
-  if ((rc = coop_result(coop, body2(), err, errcap))) return rc;
-  if (lead) { memset(out.p, 0, 64); rc = out.commit(err, errcap); }
-  else { out.unmap(); out.committed = true; }
-  return coop_result(coop, rc, err, errcap);
+  return file_call(dist_state().on, combined_fn, LF.acc_size, [] { return (int32_t)SSO_OK; },
+      [&](uint8_t* out) -> int32_t {
+        int32_t rc;
+        std::vector<RVec> vecs;
+        for (uint64_t k = 0; k < nchunks; k++) {
+          sso_p1_params_t pk = *p;
+          pk.contribution_mode = SSO_MODE_CHUNKED; pk.chunk_index = k;
+          P1Layout L;
+          if ((rc = p1_layout(&pk, L, err, errcap))) return rc;
+          ins[k].reset(new MappedFile());
+          if ((rc = ins[k]->open_ro(names[k].c_str(), err, errcap))) return rc;
+          if (ins[k]->len != L.contrib_size) { set_err(err, errcap, "The size of response file %s should be correct: %zu != %llu", names[k].c_str(), ins[k]->len, (unsigned long long)L.contrib_size); return SSO_E_ARG; }
+          const uint64_t counts[5] = {L.g1n, L.on, L.on, L.on, k == 0 ? 1ull : 0ull};       // beta_g2 is taken from the first chunk
+          for (int v = 0; v < 5; v++) {
+            if (counts[v] == 0) continue;
+            const size_t usz = point_size(L.cs, groups[v], 0);
+            vecs.push_back({groups[v], ins[k]->p + L.off_c[v], 1, counts[v], out + LF.off_u[v] + (v == 4 ? 0 : L.start * usz), 0, 0,
+                            CHECK_NO, 0, 0, vnames[v]});
+          }
+        }
+        Participants P;
+        if ((rc = resolve_participants(devices, ndev, device, true, P, err, errcap))) return rc;
+        return stream_reencode(ops, LF.cs, vecs, p->batch_size, nullptr, 0, P, nullptr, err, errcap);
+      },
+      [](Outputs&, uint8_t* out) { memset(out, 0, 64); return (int32_t)SSO_OK; }, err, errcap);
 }
 
 // phase1_cli::transform_ratios(response_fn, check_input, params) — reference src/bin/verify_transcript.rs:646-653, 811-822,
@@ -1183,17 +1135,6 @@ int32_t sso_p1_verify_ratios_file(const sso_p1_params_t* p, const char* combined
 // ---------------------------------------------------------------------------------------------
 namespace {
 
-const uint32_t* fr_modulus_host(uint32_t curve, int& L) {
-  switch (curve) {
-    case SSO_CURVE_BLS12_377: L = P_r253::L; return P_r253::host_p();
-    case SSO_CURVE_BW6_761: L = P_q377::L; return P_q377::host_p();
-    case SSO_CURVE_MNT4_753: L = P_q6::L; return P_q6::host_p();
-    case SSO_CURVE_MNT6_753: L = P_q4::L; return P_q4::host_p();
-  }
-  L = 0;
-  return nullptr;
-}
-
 // a^-1 mod p on canonical little-endian limbs (binary extended Euclid; p odd, 0 < a < p) — one inversion per contribution
 bool host_mod_inverse(const uint32_t* a, const uint32_t* p, int L, uint32_t* out) {
   auto is_zero = [&](const std::vector<uint32_t>& x) { for (uint32_t w : x) if (w) return false; return true; };
@@ -1226,8 +1167,7 @@ int scalar_mul_one(Ctx& c, const CurveOps* ops, const CurveSizes& cs, uint32_t g
   uint32_t *d_status, *d_table;
   if ((rc = c.alloc((void**)&d_in, isz))) return rc;
   if ((rc = c.alloc((void**)&d_out, usz))) return rc;
-  if ((rc = c.alloc((void**)&d_status, STATUS_BYTES))) return rc;
-  CUDA_TRY(cudaMemsetAsync(d_status, 0, STATUS_BYTES, c.s[0]));
+  if ((rc = status_buffer(c, &d_status, 0, false, err, errcap))) return rc;
   CUDA_TRY(cudaMemcpyAsync(d_in, pt, isz, cudaMemcpyHostToDevice, c.s[0]));
   std::vector<uint8_t> one(ops->fr_bytes, 0);
   one[0] = 1;
@@ -1281,11 +1221,11 @@ int32_t sso_p2_contribute_buf(uint32_t curve, const uint8_t* challenge, size_t c
   KeygenState keys;
   if ((rc = keygen_stage1(c, 0, ops, cs, seed32, 1, keys, delta.data(), err, errcap))) return rc;
   if ((rc = keygen_collect_g1(c, 0, cs, keys, err, errcap))) return rc;
-  int L;
-  const uint32_t* pmod = fr_modulus_host(curve, L);
-  std::vector<uint32_t> dw(L, 0), iw(L, 0);
+  FftDomain fr;                                             // the scalar field's modulus
+  fft_domain(curve, fr);
+  std::vector<uint32_t> dw(fr.L, 0), iw(fr.L, 0);
   memcpy(dw.data(), delta.data(), cs.fr);
-  if (!host_mod_inverse(dw.data(), pmod, L, iw.data())) { set_err(err, errcap, "delta is zero"); return SSO_E_INPUT; }
+  if (!host_mod_inverse(dw.data(), fr.modulus, (int)fr.L, iw.data())) { set_err(err, errcap, "delta is zero"); return SSO_E_INPUT; }
   std::vector<uint8_t> delta_inv(cs.fr);
   memcpy(delta_inv.data(), iw.data(), cs.fr);
   uint8_t transcript[64];
@@ -1352,7 +1292,7 @@ int32_t sso_p2_verify_buf(uint32_t curve, const uint8_t* challenge, size_t chall
     uint8_t* d_pk;
     uint32_t* d_status;
     if ((rc = c.alloc((void**)&d_pk, vr.contrib_size))) return rc;
-    if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
+    if ((rc = status_buffer(c, &d_status, 0, true, err, errcap))) return rc;
     CUDA_TRY(cudaMemcpyAsync(d_pk, pk, vr.contrib_size, cudaMemcpyHostToDevice, c.s[0]));
     if ((rc = ops->reencode(c, 0, GROUP_G1, d_pk, 0, 3, nullptr, 0, CHECK_FULL, 1, nullptr, d_status, err, errcap))) return rc;
     if ((rc = ops->reencode(c, 0, GROUP_G2, d_pk + 3 * cs.g1u, 0, 1, nullptr, 0, CHECK_FULL, 1, nullptr, d_status, err, errcap))) return rc;
@@ -1378,24 +1318,17 @@ int32_t sso_p2_verify_buf(uint32_t curve, const uint8_t* challenge, size_t chall
     const uint64_t n = qb[q]->n;
     if (n == 0) continue;
     if (n > (1ull << 24)) return reject("query longer than 2^24 elements");
-    uint8_t *d_b, *d_a, *d_pair;
-    uint32_t *d_status, *d_aff_b, *d_aff_a;
-    if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
+    uint8_t *d_b, *d_a;
+    uint32_t* d_status;
+    if ((rc = status_buffer(c, &d_status, 0, true, err, errcap))) return rc;
     if ((rc = c.alloc((void**)&d_b, n * cs.g1u))) return rc;
     if ((rc = c.alloc((void**)&d_a, n * cs.g1u))) return rc;
-    if ((rc = c.alloc((void**)&d_aff_b, n * ops->aff_words[0] * 4))) return rc;
-    if ((rc = c.alloc((void**)&d_aff_a, n * ops->aff_words[0] * 4))) return rc;
-    if ((rc = c.alloc((void**)&d_pair, 2 * cs.g1u))) return rc;
     CUDA_TRY(cudaMemcpyAsync(d_b, challenge + qb[q]->off, n * cs.g1u, cudaMemcpyHostToDevice, c.s[0]));
     CUDA_TRY(cudaMemcpyAsync(d_a, new_challenge + qa[q]->off, n * cs.g1u, cudaMemcpyHostToDevice, c.s[0]));
-    if ((rc = ops->reencode(c, 0, GROUP_G1, d_b, 0, n, nullptr, 0, CHECK_NO, 0, d_aff_b, d_status, err, errcap))) return rc;
-    if ((rc = ops->reencode(c, 0, GROUP_G1, d_a, 0, n, nullptr, 0, CHECK_NO, 0, d_aff_a, d_status, err, errcap))) return rc;
     const uint64_t tweak[4] = {TWEAK_P2_VERIFY | (uint64_t)q, n, 0, 0};
-    if ((rc = ops->msm_pairs(c, 0, GROUP_G1, d_aff_b, d_aff_a, n, rlc_seed32, tweak, d_pair, err, errcap))) return rc;
     pairs[q].resize(2 * cs.g1u);
-    CUDA_TRY(cudaMemcpyAsync(pairs[q].data(), d_pair, 2 * cs.g1u, cudaMemcpyDeviceToHost, c.s[0]));
-    CUDA_TRY(cudaStreamSynchronize(c.s[0]));
-    if ((rc = check_status(c, d_status, "query", err, errcap))) return rc == SSO_E_INPUT ? SSO_E_VERIFY : rc;
+    if ((rc = pair_to_host(c, ops, GROUP_G1, cs.g1u, n, {d_b, 0, CHECK_NO, 0}, {d_a, 0, CHECK_NO, 0}, rlc_seed32, tweak, d_status, "query",
+                           pairs[q].data(), err, errcap))) return rc == SSO_E_INPUT ? SSO_E_VERIFY : rc;
     add_check(checks, qn[q], pairs[q].data(), pairs[q].data() + cs.g1u, cs.g1u, new_challenge + vn.delta_g2, challenge + vc.delta_g2, cs.g2u);
   }
   return run_checks(c, ops, checks, err, errcap);
@@ -1408,22 +1341,19 @@ int32_t sso_p2_contribute_file(uint32_t curve, const char* challenge_fn, const c
                                char* err, size_t errcap) {
   (void)batch_exp_mode;
   if (!challenge_fn || !challenge_hash_fn || !response_fn || !response_hash_fn || !seed32) { set_err(err, errcap, "null argument"); return SSO_E_ARG; }
-  MappedFile in, out;
+  MappedFile in;
+  Outputs outs;
+  uint8_t* out;
   int rc;
   if ((rc = in.open_ro(challenge_fn, err, errcap))) return rc;
   size_t need = 0;
   rc = sso_p2_contribute_buf(curve, in.p, in.len, nullptr, 0, &need, seed32, check_input, device, err, errcap);
   if (rc != SSO_E_ARG || need == 0) return rc ? rc : SSO_E_ARG;
-  if ((rc = out.create(response_fn, need, true, err, errcap))) return rc;
-  if ((rc = sso_p2_contribute_buf(curve, in.p, in.len, out.p, out.len, &need, seed32, check_input, device, err, errcap))) return rc;
-  uint8_t h[64];
-  std::vector<SmallFile> small;
-  blake2b_512(in.p, in.len, h);
-  if ((rc = write_small(small, challenge_hash_fn, h, 64, err, errcap))) return rc;
-  blake2b_512(out.p, out.len, h);
-  if ((rc = write_small(small, response_hash_fn, h, 64, err, errcap))) { discard_small(small); return rc; }
-  if ((rc = out.commit(err, errcap))) { discard_small(small); return rc; }
-  return commit_small(small, err, errcap);
+  if ((rc = outs.create_mapped(response_fn, need, true, &out, err, errcap))) return rc;
+  if ((rc = sso_p2_contribute_buf(curve, in.p, in.len, out, need, &need, seed32, check_input, device, err, errcap))) return rc;
+  if ((rc = outs.write_hash(challenge_hash_fn, in.p, in.len, err, errcap))) return rc;
+  if ((rc = outs.write_hash(response_hash_fn, out, need, err, errcap))) return rc;
+  return outs.commit(err, errcap);
 }
 
 // phase2_cli::verify::<P>(challenge_fn, challenge_hash_fn, check_input, response_fn, response_hash_fn, check_output, new_challenge_fn,
@@ -1433,26 +1363,21 @@ int32_t sso_p2_verify_file(uint32_t curve, const char* challenge_fn, const char*
                            uint32_t subgroup_check_mode, uint32_t verify_full, int device, char* err, size_t errcap) {
   (void)verify_full;                                       // this container is always the full parameter set
   if (!challenge_fn || !challenge_hash_fn || !response_fn || !response_hash_fn || !new_challenge_fn || !new_challenge_hash_fn) { set_err(err, errcap, "null argument"); return SSO_E_ARG; }
-  MappedFile ch, resp, out;
+  MappedFile ch, resp;
+  Outputs outs;
+  uint8_t* out;
   int rc;
   if ((rc = ch.open_ro(challenge_fn, err, errcap))) return rc;
   if ((rc = resp.open_ro(response_fn, err, errcap))) return rc;
   size_t need = 0;
   rc = sso_p2_verify_buf(curve, ch.p, ch.len, resp.p, resp.len, nullptr, 0, &need, check_input, check_output, subgroup_check_mode, nullptr, device, err, errcap);
   if (rc != SSO_E_ARG || need == 0) return rc ? rc : SSO_E_ARG;
-  if ((rc = out.create(new_challenge_fn, need, true, err, errcap))) return rc;
-  if ((rc = sso_p2_verify_buf(curve, ch.p, ch.len, resp.p, resp.len, out.p, out.len, &need, check_input, check_output, subgroup_check_mode, nullptr, device, err, errcap))) return rc;
-  uint8_t h[64];
-  std::vector<SmallFile> small;
-  auto fail = [&](int32_t rc) { discard_small(small); return rc; };
-  blake2b_512(ch.p, ch.len, h);
-  if ((rc = write_small(small, challenge_hash_fn, h, 64, err, errcap))) return fail(rc);
-  blake2b_512(resp.p, resp.len, h);
-  if ((rc = write_small(small, response_hash_fn, h, 64, err, errcap))) return fail(rc);
-  blake2b_512(out.p, out.len, h);
-  if ((rc = write_small(small, new_challenge_hash_fn, h, 64, err, errcap))) return fail(rc);
-  if ((rc = out.commit(err, errcap))) return fail(rc);
-  return commit_small(small, err, errcap);
+  if ((rc = outs.create_mapped(new_challenge_fn, need, true, &out, err, errcap))) return rc;
+  if ((rc = sso_p2_verify_buf(curve, ch.p, ch.len, resp.p, resp.len, out, need, &need, check_input, check_output, subgroup_check_mode, nullptr, device, err, errcap))) return rc;
+  if ((rc = outs.write_hash(challenge_hash_fn, ch.p, ch.len, err, errcap))) return rc;
+  if ((rc = outs.write_hash(response_hash_fn, resp.p, resp.len, err, errcap))) return rc;
+  if ((rc = outs.write_hash(new_challenge_hash_fn, out, need, err, errcap))) return rc;
+  return outs.commit(err, errcap);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1470,7 +1395,7 @@ int32_t sso_group_fft_dev(uint32_t curve, uint32_t group, const void* d_in, uint
   if (rc) return rc;
   if (group > 1 || !d_in || !d_out) { set_err(err, errcap, "unknown group %u or null buffer", group); return SSO_E_ARG; }
   uint32_t* d_status;
-  if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
+  if ((rc = status_buffer(c, &d_status, 0, true, err, errcap))) return rc;
   CurveSizes cs;
   curve_sizes(curve, cs);
   const uint8_t* src = (const uint8_t*)d_in;
@@ -1520,14 +1445,16 @@ int32_t sso_p2_prepare_file(const char* phase2_fn, const char* response_fn, uint
   int log_m;
   int rc = p2prep_check(p, phase2_size, L, d, log_m, err, errcap);
   if (rc) return rc;
-  MappedFile in, out;
+  MappedFile in;
+  Outputs outs;
+  uint8_t* out;
   if ((rc = in.open_ro(response_fn, err, errcap))) return rc;
   size_t need = 0;
   rc = sso_p2_prepare_buf(p, in.p, in.len, phase2_size, nullptr, 0, &need, device, err, errcap);
   if (rc != SSO_E_ARG || need == 0) return rc ? rc : SSO_E_ARG;
-  if ((rc = out.create(phase2_fn, need, true, err, errcap))) return rc;
-  if ((rc = sso_p2_prepare_buf(p, in.p, in.len, phase2_size, out.p, out.len, &need, device, err, errcap))) return rc;
-  return out.commit(err, errcap);
+  if ((rc = outs.create_mapped(phase2_fn, need, true, &out, err, errcap))) return rc;
+  if ((rc = sso_p2_prepare_buf(p, in.p, in.len, phase2_size, out, need, &need, device, err, errcap))) return rc;
+  return outs.commit(err, errcap);
 }
 
 int32_t sso_imad_peak(int device, int variant, double* macs_per_s, char* err, size_t errcap) {
@@ -1573,7 +1500,7 @@ int32_t sso_test_field_mul(uint32_t field, const uint8_t* a, const uint8_t* b, u
   if ((rc = c.alloc((void**)&d_a, bytes))) return rc;
   if ((rc = c.alloc((void**)&d_b, bytes))) return rc;
   if ((rc = c.alloc((void**)&d_o, bytes))) return rc;
-  if ((rc = status_buffer(c, &d_status, err, errcap))) return rc;
+  if ((rc = status_buffer(c, &d_status, 0, true, err, errcap))) return rc;
   CUDA_TRY(cudaMemcpyAsync(d_a, a, bytes, cudaMemcpyHostToDevice, c.s[0]));
   CUDA_TRY(cudaMemcpyAsync(d_b, b, bytes, cudaMemcpyHostToDevice, c.s[0]));
   uint32_t g = div_up(n, 128);

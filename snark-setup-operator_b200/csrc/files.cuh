@@ -7,11 +7,21 @@
 #include <sys/stat.h>
 #include <fcntl.h>
 #include <unistd.h>
+#include <deque>
 #include <string>
 #include <mutex>
 #include <vector>
 
+#include "blake2b.h"
+
 namespace sso {
+
+// create_new on the final name: an output that already exists is an error
+inline int refuse_existing(const char* fn, char* err, size_t errcap) {
+  struct stat st;
+  if (stat(fn, &st) == 0) { set_err(err, errcap, "cannot create %s (outputs must not exist)", fn); return SSO_E_IO; }
+  return SSO_OK;
+}
 
 struct MappedFile {
   uint8_t* p = nullptr;
@@ -47,8 +57,8 @@ struct MappedFile {
     owner = is_owner;
     len = size;
     if (owner) {
-      struct stat st;
-      if (stat(fn, &st) == 0) { set_err(err, errcap, "cannot create %s (outputs must not exist)", fn); return SSO_E_IO; }
+      int rc = refuse_existing(fn, err, errcap);
+      if (rc) return rc;
       fd = ::open(tmp.c_str(), O_RDWR | O_CREAT | O_EXCL, 0644);
       if (fd < 0) { set_err(err, errcap, "cannot create %s (outputs must not exist)", tmp.c_str()); return SSO_E_IO; }
       if (ftruncate(fd, (off_t)size) != 0) { set_err(err, errcap, "cannot size %s to %zu bytes", tmp.c_str(), size); return SSO_E_IO; }
@@ -130,33 +140,63 @@ inline int read_file_into(const char* path, uint8_t* dst, size_t expect, char* e
   return SSO_OK;
 }
 
-// small outputs (the 64-byte hash files): written whole under a temporary name, renamed by commit_small_files
-struct SmallFile { std::string path, tmp; };
-inline int write_small(std::vector<SmallFile>& pending, const char* path, const uint8_t* data, size_t len, char* err, size_t errcap) {
-  struct stat st;
-  if (stat(path, &st) == 0) { set_err(err, errcap, "cannot create %s (outputs must not exist)", path); return SSO_E_IO; }
-  SmallFile f{path, std::string(path) + ".sso-partial"};
-  int fd = ::open(f.tmp.c_str(), O_WRONLY | O_CREAT | O_EXCL, 0644);
-  if (fd < 0) { set_err(err, errcap, "cannot create %s (outputs must not exist)", f.tmp.c_str()); return SSO_E_IO; }
-  size_t put = 0;
-  while (put < len) {
-    ssize_t w = write(fd, data + put, len - put);
-    if (w <= 0) { ::close(fd); unlink(f.tmp.c_str()); set_err(err, errcap, "short write on %s", f.tmp.c_str()); return SSO_E_IO; }
-    put += (size_t)w;
+// Every output of one file call.  Each is created under <name>.sso-partial (create_new semantics on both names): the mapped
+// outputs the call fills in place, and the small files written whole (the hash files; in the chunk-sized paths also the
+// response or new challenge).  commit() renames them into place, mapped outputs first, then the small files in the order
+// they were written; whatever is not committed is removed on destruction.  A mapped output created by a non-owner (another
+// rank of the process group mapping the owner's partial file) is only detached from: never renamed, never removed.
+struct Outputs {
+  std::deque<MappedFile> mapped;
+  std::vector<std::string> small;                // final names
+  bool committed = false;
+
+  Outputs() = default;
+  Outputs(const Outputs&) = delete;
+  Outputs& operator=(const Outputs&) = delete;
+
+  int create_mapped(const char* fn, size_t size, bool owner, uint8_t** p, char* err, size_t errcap) {
+    mapped.emplace_back();
+    int rc = mapped.back().create(fn, size, owner, err, errcap);
+    *p = mapped.back().p;
+    return rc;
   }
-  ::close(fd);
-  pending.push_back(f);
-  return SSO_OK;
-}
-inline void discard_small(std::vector<SmallFile>& pending) {
-  for (auto& f : pending) unlink(f.tmp.c_str());
-  pending.clear();
-}
-inline int commit_small(std::vector<SmallFile>& pending, char* err, size_t errcap) {
-  for (auto& f : pending)
-    if (rename(f.tmp.c_str(), f.path.c_str()) != 0) { set_err(err, errcap, "cannot rename %s to %s", f.tmp.c_str(), f.path.c_str()); discard_small(pending); return SSO_E_IO; }
-  pending.clear();
-  return SSO_OK;
-}
+  int write_whole(const char* fn, const uint8_t* data, size_t len, char* err, size_t errcap) {
+    int rc = refuse_existing(fn, err, errcap);
+    if (rc) return rc;
+    const std::string tmp = std::string(fn) + ".sso-partial";
+    int fd = ::open(tmp.c_str(), O_WRONLY | O_CREAT | O_EXCL, 0644);
+    if (fd < 0) { set_err(err, errcap, "cannot create %s (outputs must not exist)", tmp.c_str()); return SSO_E_IO; }
+    size_t put = 0;
+    while (put < len) {
+      ssize_t w = write(fd, data + put, len - put);
+      if (w <= 0) { ::close(fd); unlink(tmp.c_str()); set_err(err, errcap, "short write on %s", tmp.c_str()); return SSO_E_IO; }
+      put += (size_t)w;
+    }
+    ::close(fd);
+    small.push_back(fn);
+    return SSO_OK;
+  }
+  // the 64 raw bytes of Blake2b-512(data)
+  int write_hash(const char* fn, const uint8_t* data, size_t len, char* err, size_t errcap) {
+    uint8_t h[64];
+    blake2b_512(data, len, h);
+    return write_whole(fn, h, 64, err, errcap);
+  }
+  int commit(char* err, size_t errcap) {
+    int rc;
+    for (MappedFile& m : mapped)
+      if ((rc = m.commit(err, errcap))) return rc;
+    for (const std::string& fn : small) {
+      const std::string tmp = fn + ".sso-partial";
+      if (rename(tmp.c_str(), fn.c_str()) != 0) { set_err(err, errcap, "cannot rename %s to %s", tmp.c_str(), fn.c_str()); return SSO_E_IO; }
+    }
+    committed = true;
+    return SSO_OK;
+  }
+  ~Outputs() {
+    if (!committed)
+      for (const std::string& fn : small) unlink((fn + ".sso-partial").c_str());
+  }
+};
 
 }  // namespace sso

@@ -6,9 +6,6 @@
 #include <thread>
 #include <mutex>
 #include <atomic>
-#include <fcntl.h>
-#include <sys/stat.h>
-#include <unistd.h>
 
 #include "blake2b.h"
 #include "curve_ops.cuh"
@@ -16,34 +13,11 @@
 
 namespace sso {
 
-// ---- small file helpers (the reference CLI mmaps inputs and creates outputs with create_new) ----
-inline int read_file(const char* path, std::vector<uint8_t>& out, char* err, size_t errcap) {
-  int fd = open(path, O_RDONLY);
-  if (fd < 0) { set_err(err, errcap, "cannot open %s", path); return SSO_E_IO; }
-  struct stat st;
-  if (fstat(fd, &st) != 0) { close(fd); set_err(err, errcap, "cannot stat %s", path); return SSO_E_IO; }
-  out.resize((size_t)st.st_size);
-  size_t got = 0;
-  while (got < out.size()) {
-    ssize_t r = read(fd, out.data() + got, out.size() - got);
-    if (r <= 0) { close(fd); set_err(err, errcap, "short read on %s", path); return SSO_E_IO; }
-    got += (size_t)r;
-  }
-  close(fd);
-  return SSO_OK;
-}
-inline int write_new_file(const char* path, const uint8_t* data, size_t len, char* err, size_t errcap) {
-  int fd = open(path, O_WRONLY | O_CREAT | O_EXCL, 0644);
-  if (fd < 0) { set_err(err, errcap, "cannot create %s (outputs must not exist)", path); return SSO_E_IO; }
-  size_t put = 0;
-  while (put < len) {
-    ssize_t w = write(fd, data + put, len - put);
-    if (w <= 0) { close(fd); unlink(path); set_err(err, errcap, "short write on %s", path); return SSO_E_IO; }
-    put += (size_t)w;
-  }
-  close(fd);
-  return SSO_OK;
-}
+// joins the thread when the scope ends, on an early return too
+struct JoinOnExit {
+  std::thread& t;
+  ~JoinOnExit() { if (t.joinable()) t.join(); }
+};
 
 // ---- key generation (Phase1::key_generation) ---------------------------------------------------
 // seed32: ChaCha20 seed of the contributor RNG; digest64: Blake2b(challenge).
@@ -231,7 +205,7 @@ inline int verify_chunk_host(Ctx& c, const CurveOps* ops, const P1Layout& L, uin
   // the response hash has its own thread: at accumulator scale (a gigabyte and more) the two sequential Blake2b passes are
   // the critical path of the call (~1 GB/s each)
   std::thread resp_hasher([&] { blake2b_512(response, L.contrib_size, side.resp_hash); });
-  struct Joiner0 { std::thread& t; ~Joiner0() { if (t.joinable()) t.join(); } } joiner0{resp_hasher};
+  JoinOnExit join_resp_hasher{resp_hasher};
   std::thread side_thread([&] {
     char* err = side.err; size_t errcap = sizeof side.err;
     side.rc = [&]() -> int {
@@ -245,10 +219,9 @@ inline int verify_chunk_host(Ctx& c, const CurveOps* ops, const P1Layout& L, uin
       uint8_t *d_pk, *d_g2s;
       uint32_t *d_status, *d_seeds2;
       if ((rc = c2.alloc((void**)&d_pk, L.pk_size, si))) return rc;
-      if ((rc = c2.alloc((void**)&d_status, STATUS_BYTES, si))) return rc;
+      if ((rc = status_buffer(c2, &d_status, si, false, err, errcap))) return rc;
       if ((rc = c2.alloc((void**)&d_seeds2, 96, si))) return rc;
       if ((rc = c2.alloc((void**)&d_g2s, 3 * g2u, si))) return rc;
-      CUDA_TRY(cudaMemsetAsync(d_status, 0, STATUS_BYTES, c2.s[si]));
       CUDA_TRY(cudaMemcpyAsync(d_pk, pk, L.pk_size, cudaMemcpyHostToDevice, c2.s[si]));
       if ((rc = ops->reencode(c2, si, GROUP_G1, d_pk, 0, 6, nullptr, 0, CHECK_FULL, 1, nullptr, d_status, err, errcap))) return rc;
       if ((rc = ops->reencode(c2, si, GROUP_G2, d_pk + 6 * g1u, 0, 3, nullptr, 0, CHECK_FULL, 1, nullptr, d_status, err, errcap))) return rc;
@@ -271,7 +244,7 @@ inline int verify_chunk_host(Ctx& c, const CurveOps* ops, const P1Layout& L, uin
       return SSO_OK;
     }();
   });
-  struct Joiner { std::thread& t; ~Joiner() { if (t.joinable()) t.join(); } } joiner{side_thread};
+  JoinOnExit join_side_thread{side_thread};
   std::vector<uint8_t> pairs[4];
   if (!P) {
     // 1. decode + check the response vectors on the device, producing the new challenge image
@@ -279,8 +252,7 @@ inline int verify_chunk_host(Ctx& c, const CurveOps* ops, const P1Layout& L, uin
     uint32_t* d_status;
     if ((rc = c.alloc((void**)&d_resp, L.contrib_size))) return rc;
     if ((rc = c.alloc((void**)&d_new, L.acc_size))) return rc;
-    if ((rc = c.alloc((void**)&d_status, STATUS_BYTES))) return rc;
-    CUDA_TRY(cudaMemsetAsync(d_status, 0, STATUS_BYTES, c.s[0]));
+    if ((rc = status_buffer(c, &d_status, 0, false, err, errcap))) return rc;
     CUDA_TRY(cudaMemcpyAsync(d_resp, response, L.contrib_size, cudaMemcpyHostToDevice, c.s[0]));
     CUDA_TRY(cudaStreamSynchronize(c.s[0]));
     uint32_t* d_aff[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
@@ -315,7 +287,7 @@ inline int verify_chunk_host(Ctx& c, const CurveOps* ops, const P1Layout& L, uin
     for (int v = 0; v < 4; v++) {
       if (!d_aff[v]) continue;
       int si = stream_of[v];
-      size_t usz = groups[v] == GROUP_G1 ? g1u : g2u;
+      const size_t usz = point_size(L.cs, groups[v], 0);
       const uint64_t tweak[4] = {TWEAK_P1_VERIFY | (uint64_t)v, chunk_index, 0, 0};
       if ((rc = c.alloc((void**)&d_pairs[v], 2 * usz, si))) return rc;
       if ((rc = ops->msm_pairs(c, si, groups[v], d_aff[v], d_aff[v] + ops->aff_words[groups[v]], counts[v] - 1, rlc_seed32, tweak,
@@ -328,8 +300,7 @@ inline int verify_chunk_host(Ctx& c, const CurveOps* ops, const P1Layout& L, uin
     if (check_input != CHECK_NO) {
       uint8_t* d_ch;
       if ((rc = c.alloc((void**)&d_ch, L.acc_size))) return rc;
-      if ((rc = c.alloc((void**)&d_status_in, STATUS_BYTES))) return rc;
-      CUDA_TRY(cudaMemsetAsync(d_status_in, 0, STATUS_BYTES, c.s[0]));
+      if ((rc = status_buffer(c, &d_status_in, 0, false, err, errcap))) return rc;
       CUDA_TRY(cudaMemcpyAsync(d_ch, challenge, L.acc_size, cudaMemcpyHostToDevice, c.s[0]));
       for (int v = 0; v < 5; v++) {
         if (counts[v] == 0) continue;
@@ -343,7 +314,7 @@ inline int verify_chunk_host(Ctx& c, const CurveOps* ops, const P1Layout& L, uin
     CUDA_TRY(cudaMemcpy(new_challenge + 64, d_new + 64, L.acc_size - 64, cudaMemcpyDeviceToHost));
     for (int v = 0; v < 4; v++) {
       if (!d_pairs[v]) continue;
-      pairs[v].resize(2 * (groups[v] == GROUP_G1 ? g1u : g2u));
+      pairs[v].resize(2 * point_size(L.cs, groups[v], 0));
       CUDA_TRY(cudaMemcpy(pairs[v].data(), d_pairs[v], pairs[v].size(), cudaMemcpyDeviceToHost));
     }
     c.mark("verify: results D2H");

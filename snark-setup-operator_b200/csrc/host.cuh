@@ -240,6 +240,14 @@ inline int upload_scalar(Ctx& c, const uint8_t* bytes, size_t nbytes, size_t nwo
 
 // status words written by kernels: [0] code, [1] element index inside its vector, [2] vector index
 static constexpr size_t STATUS_BYTES = 16;
+// a zeroed status buffer on stream si; `sync` drains that stream before the call goes on
+inline int status_buffer(Ctx& c, uint32_t** d_status, int si, bool sync, char* err, size_t errcap) {
+  int rc = c.alloc((void**)d_status, STATUS_BYTES, si);
+  if (rc) return rc;
+  CUDA_TRY(cudaMemsetAsync(*d_status, 0, STATUS_BYTES, c.s[si]));
+  if (sync) CUDA_TRY(cudaStreamSynchronize(c.s[si]));
+  return SSO_OK;
+}
 inline int check_status(Ctx& c, uint32_t* d_status, const char* what, char* err, size_t errcap) {
   uint32_t h[4] = {0, 0, 0, 0};
   CUDA_TRY(cudaMemcpy(h, d_status, STATUS_BYTES, cudaMemcpyDeviceToHost));

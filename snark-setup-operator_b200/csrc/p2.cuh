@@ -44,8 +44,8 @@ inline void wr_u32be(uint8_t* p, uint32_t v) { p[0] = (uint8_t)(v >> 24); p[1] =
 
 inline int p2_parse(const uint8_t* buf, size_t len, bool compressed, const CurveSizes& cs, P2View& v, char* err, size_t errcap) {
   v.compressed = compressed;
-  v.g1 = compressed ? cs.g1c : cs.g1u;
-  v.g2 = compressed ? cs.g2c : cs.g2u;
+  v.g1 = point_size(cs, GROUP_G1, compressed);
+  v.g2 = point_size(cs, GROUP_G2, compressed);
   v.contrib_size = 3 * cs.g1u + cs.g2u + 64;
   size_t o = 0;
   auto need = [&](size_t n) { return o + n <= len; };
@@ -54,7 +54,7 @@ inline int p2_parse(const uint8_t* buf, size_t len, bool compressed, const Curve
     if (!need(8)) return false;
     f.n = rd_u64le(buf + o); o += 8;
     f.off = o; f.group = group;
-    size_t sz = group == GROUP_G1 ? v.g1 : v.g2;
+    const size_t sz = point_size(cs, group, compressed);
     if (f.n > (len - o) / sz) return false;
     o += f.n * sz;
     return true;
@@ -75,7 +75,7 @@ inline int p2_parse(const uint8_t* buf, size_t len, bool compressed, const Curve
 
 // size of the container with the element counts of `v` in the other encoding and `extra` more contributions
 inline size_t p2_size(const P2View& v, const CurveSizes& cs, bool compressed, uint32_t extra) {
-  size_t g1 = compressed ? cs.g1c : cs.g1u, g2 = compressed ? cs.g2c : cs.g2u;
+  const size_t g1 = point_size(cs, GROUP_G1, compressed), g2 = point_size(cs, GROUP_G2, compressed);
   uint64_t n1 = v.gamma_abc.n + v.a_query.n + v.b_g1_query.n + v.h_query.n + v.l_query.n;
   return (3 + n1) * g1 + (3 + v.b_g2_query.n) * g2 + 6 * 8 + 64 + 4 + (size_t)(v.n_contrib + extra) * v.contrib_size;
 }
@@ -110,8 +110,7 @@ inline int p2_transform(Ctx& c, const CurveOps* ops, const CurveSizes& cs, const
   std::vector<uint8_t> one(ops->fr_bytes, 0);
   one[0] = 1;
   uint32_t* d_status;
-  if ((rc = c.alloc((void**)&d_status, STATUS_BYTES))) return rc;
-  CUDA_TRY(cudaMemsetAsync(d_status, 0, STATUS_BYTES, c.s[0]));
+  if ((rc = status_buffer(c, &d_status, 0, false, err, errcap))) return rc;
   const uint64_t SEG = 1ull << 22;
   for (const P2Item& it : items) {
     const size_t isz = point_size(cs, it.group, vi.compressed), osz = point_size(cs, it.group, out_compressed);

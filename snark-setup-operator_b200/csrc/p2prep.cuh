@@ -92,8 +92,7 @@ inline int p2_prepare(Ctx& c, const CurveOps* ops, const P1Layout& L, const FftD
   static const uint32_t grp[5] = {GROUP_G1, GROUP_G2, GROUP_G1, GROUP_G1, GROUP_G2};
   uint8_t* d_in[5];
   uint32_t* d_status;
-  if ((rc = c.alloc((void**)&d_status, STATUS_BYTES))) return rc;
-  CUDA_TRY(cudaMemsetAsync(d_status, 0, STATUS_BYTES, c.s[0]));
+  if ((rc = status_buffer(c, &d_status, 0, false, err, errcap))) return rc;
   for (int v = 0; v < 5; v++) {
     const size_t bytes = cnt[v] * point_size(cs, grp[v], 0);
     if ((rc = c.alloc((void**)&d_in[v], bytes))) return rc;

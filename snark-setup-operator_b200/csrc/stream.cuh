@@ -236,8 +236,7 @@ inline int sum_points_host(Ctx& c, const CurveOps* ops, uint32_t group, size_t u
   int rc;
   if ((rc = c.alloc((void**)&d_in, cnt * usz))) return rc;
   if ((rc = c.alloc((void**)&d_out, usz))) return rc;
-  if ((rc = c.alloc((void**)&d_status, STATUS_BYTES))) return rc;
-  CUDA_TRY(cudaMemsetAsync(d_status, 0, STATUS_BYTES, c.s[0]));
+  if ((rc = status_buffer(c, &d_status, 0, false, err, errcap))) return rc;
   CUDA_TRY(cudaMemcpyAsync(d_in, pts, cnt * usz, cudaMemcpyHostToDevice, c.s[0]));
   if ((rc = ops->points_sum(c, 0, group, d_in, (uint32_t)cnt, d_out, d_status, err, errcap))) return rc;
   CUDA_TRY(cudaMemcpyAsync(out, d_out, usz, cudaMemcpyDeviceToHost, c.s[0]));
@@ -302,8 +301,7 @@ inline int exchange_and_sum(const CurveOps* ops, const CurveSizes& cs, const Par
       uint32_t* d_status;
       if ((rc = c.alloc((void**)&d_pts, vusz[v] * total))) return rc;
       if ((rc = c.alloc((void**)&d_out, vusz[v]))) return rc;
-      if ((rc = c.alloc((void**)&d_status, STATUS_BYTES))) return rc;
-      CUDA_TRY(cudaMemsetAsync(d_status, 0, STATUS_BYTES, c.s[0]));
+      if ((rc = status_buffer(c, &d_status, 0, false, err, errcap))) return rc;
       CUDA_TRY(cudaMemcpy2DAsync(d_pts, vusz[v], d_recv[0] + voff[v] + half * vusz[v], blob, vusz[v], total, cudaMemcpyDeviceToDevice, c.s[0]));
       if ((rc = ops->points_sum(c, 0, vecs[v].group, d_pts, (uint32_t)total, d_out, d_status, err, errcap))) return rc;
       CUDA_TRY(cudaMemcpyAsync(pairs[v].data() + half * vusz[v], d_out, vusz[v], cudaMemcpyDeviceToHost, c.s[0]));
@@ -352,8 +350,7 @@ inline int stream_reencode(const CurveOps* ops, const CurveSizes& cs, const std:
     if (r.out && (rc = c.alloc((void**)&d_out, pc.cnt * osz))) return rc;
     if (pairs_here && (rc = c.alloc((void**)&d_aff, pc.cnt * ops->aff_words[r.group] * 4))) return rc;
     if (pairs_here && (rc = c.alloc((void**)&d_pair, 2 * usz))) return rc;
-    if ((rc = c.alloc((void**)&d_status, STATUS_BYTES))) return rc;
-    CUDA_TRY(cudaMemsetAsync(d_status, 0, STATUS_BYTES, c.s[0]));
+    if ((rc = status_buffer(c, &d_status, 0, false, err, errcap))) return rc;
     CUDA_TRY(cudaMemcpyAsync(d_in, r.in + pc.lo * isz, pc.cnt * isz, cudaMemcpyHostToDevice, c.s[0]));
     if ((rc = ops->reencode(c, 0, r.group, d_in, r.in_compressed, pc.cnt, d_out, r.out_compressed, r.check, r.subgroup, d_aff, d_status, e, ec))) return rc;
     std::vector<uint8_t> pair;
@@ -447,8 +444,7 @@ inline int stream_contribute(const CurveOps* ops, const P1Layout& L, const uint8
     int rc;
     if ((rc = c.alloc((void**)&d_in, pc.cnt * usz))) return rc;
     if ((rc = c.alloc((void**)&d_out, pc.cnt * csz))) return rc;
-    if ((rc = c.alloc((void**)&d_status, STATUS_BYTES))) return rc;
-    CUDA_TRY(cudaMemsetAsync(d_status, 0, STATUS_BYTES, c.s[0]));
+    if ((rc = status_buffer(c, &d_status, 0, false, err, errcap))) return rc;
     CUDA_TRY(cudaMemcpyAsync(d_in, challenge + L.off_u[pc.vec] + pc.lo * usz, pc.cnt * usz, cudaMemcpyHostToDevice, c.s[0]));
     if (check == CHECK_FULL) {                     // CheckForCorrectness::Full on the inputs: on the curve AND in the subgroup
       if ((rc = ops->reencode(c, 0, g, d_in, 0, pc.cnt, nullptr, 0, CHECK_FULL, 1, nullptr, d_status, e, ec))) return rc;
