@@ -345,6 +345,27 @@ int32_t sso_p2_prepare_buf(const sso_p1_params_t* p, const uint8_t* accumulator,
 int32_t sso_p2_prepare_file(const char* phase2_fn, const char* response_fn, uint64_t phase2_size, const sso_p1_params_t* p, int device,
                             char* err, size_t errcap);
 
+/* The same transforms in parts: a four-step group FFT (2^log_n = parts * M points; per part a size-M FFT of the stride-`parts`
+ * subsequence and its twiddles, then per block of columns a `parts`-point FFT over the rows), with the output buffer (or file) as the
+ * exchange buffer and device memory per task of the order of one part.  They run on the devices of the calling process, never
+ * cooperatively over a process group: devices[0..ndev) (NULL / 0: `device`; device = -1: all visible); an entry may repeat, for one
+ * more worker on that device.  Every size and argument check comes before any device use.
+ *
+ * Group FFT of 2^log_n uncompressed points on HOST buffers in `parts` parts (a power of two up to 2^24, 2^log_n / parts <= 2^24; log_n up to the
+ * 2-adicity of Fr): the same transform and bytes as sso_group_fft_dev, for any parts.  in and out are 2^log_n points each and must
+ * not overlap. */
+int32_t sso_group_fft_parts_buf(uint32_t curve, uint32_t group, const uint8_t* in, size_t in_len, uint32_t log_n, uint32_t inverse,
+                                uint8_t* out, size_t out_len, uint64_t parts, const int* devices, int ndev, int device, char* err, size_t errcap);
+/* prepare_phase2 as sso_p2_prepare_buf / _file, for m up to min(2^power, 2^two-adicity) (MNT6-753 stays at 2^15), the number of parts
+ * chosen automatically: the smallest power of two that is at least the number of workers, keeps a part at 2^24 points or fewer and
+ * fits a part of the G2 vector into the free device memory of each worker at call start.  The same output bytes as
+ * sso_p2_prepare_buf wherever that accepts the size, and the same checks of every accumulator element read (SSO_E_INPUT); the first
+ * failure stops the call.  The file variant refuses an existing output (SSO_E_IO) before any device use. */
+int32_t sso_p2_prepare_devices_buf(const sso_p1_params_t* p, const uint8_t* accumulator, size_t len, uint64_t phase2_size, uint8_t* out,
+                                   size_t out_cap, size_t* out_len, const int* devices, int ndev, int device, char* err, size_t errcap);
+int32_t sso_p2_prepare_devices_file(const char* phase2_fn, const char* response_fn, uint64_t phase2_size, const sso_p1_params_t* p,
+                                    const int* devices, int ndev, int device, char* err, size_t errcap);
+
 /* setup_utils::calculate_hash (reference src/utils.rs:618-623): Blake2b-512, unkeyed. Host only. */
 int32_t sso_blake2b_512(const uint8_t* data, size_t len, uint8_t out[64]);
 

@@ -1457,6 +1457,78 @@ int32_t sso_p2_prepare_file(const char* phase2_fn, const char* response_fn, uint
   return outs.commit(err, errcap);
 }
 
+// The group FFT in parts on host buffers (p2prep.cuh parts_fft): the transform of sso_group_fft_dev, uncompressed, for any number of
+// parts and past 2^24 points, over the devices of this process.
+int32_t sso_group_fft_parts_buf(uint32_t curve, uint32_t group, const uint8_t* in, size_t in_len, uint32_t log_n, uint32_t inverse,
+                                uint8_t* out, size_t out_len, uint64_t parts, const int* devices, int ndev, int device, char* err, size_t errcap) {
+  const CurveOps* ops = ops_for(curve);
+  FftDomain d;
+  CurveSizes cs;
+  if (!ops || !fft_domain(curve, d) || !curve_sizes(curve, cs)) { set_err(err, errcap, "unknown curve %u", curve); return SSO_E_ARG; }
+  if (group > 1) { set_err(err, errcap, "unknown group %u", group); return SSO_E_ARG; }
+  if (log_n > d.two_adicity) { set_err(err, errcap, "group FFT of 2^%u points: beyond the radix-2 domain (2^%u)", log_n, d.two_adicity); return SSO_E_ARG; }
+  const int log_p = log2_exact(parts);
+  if (log_p < 0 || (uint32_t)log_p > log_n || log_n - (uint32_t)log_p > 24 || log_p > 24) {
+    set_err(err, errcap, "%llu parts of 2^%u points: a power of two up to 2^24 and the number of points, with parts of at most 2^24 points",
+            (unsigned long long)parts, log_n);
+    return SSO_E_ARG;
+  }
+  const uint64_t n = 1ull << log_n;
+  const size_t bytes = n * point_size(cs, group, 0);
+  if (!in || !out || in_len != bytes || out_len != bytes) {
+    set_err(err, errcap, "input and output must be %zu bytes each (2^%u uncompressed points)", bytes, log_n);
+    return SSO_E_ARG;
+  }
+  if (in < out + out_len && out < in + in_len) { set_err(err, errcap, "the output must not overlap the input"); return SSO_E_ARG; }
+  Participants Pt;
+  int rc = resolve_participants(devices, ndev, device, false, Pt, err, errcap);
+  if (rc) return rc;
+  std::vector<uint8_t> minv;
+  if (inverse) minv = fft_inv_size(d, log_n, ops->fr_bytes);
+  const PartsPlan pl = parts_plan(log_n, (uint32_t)log_p, inverse ? d.root_inv : d.root, d.two_adicity, inverse ? minv.data() : nullptr);
+  const PartsVec v = {group, in, out, 0};
+  return parts_fft(ops, cs, pl, &v, 1, Pt, CHECK_NO, "group FFT input", 0, nullptr, err, errcap);
+}
+
+// prepare_phase2 in parts over the devices of this process (p2prep.cuh p2_prepare_devices): the output of sso_p2_prepare_buf, for
+// every size the radix-2 domain and the accumulator allow.
+int32_t sso_p2_prepare_devices_buf(const sso_p1_params_t* p, const uint8_t* accumulator, size_t len, uint64_t phase2_size, uint8_t* out,
+                                   size_t out_cap, size_t* out_len, const int* devices, int ndev, int device, char* err, size_t errcap) {
+  if (out_len) *out_len = 0;
+  P1Layout L;
+  FftDomain d;
+  int log_m;
+  int rc = p2prep_check(p, phase2_size, L, d, log_m, err, errcap, 64);
+  if (rc) return rc;
+  if (!out_len) { set_err(err, errcap, "null out_len"); return SSO_E_ARG; }
+  if (!accumulator || len != L.acc_size) { set_err(err, errcap, "accumulator is %zu bytes, the parameters give %llu", len, (unsigned long long)L.acc_size); return SSO_E_ARG; }
+  const size_t need = p2prep_size(L.cs, phase2_size);
+  *out_len = need;
+  if (!out || out_cap < need) { set_err(err, errcap, "output buffer too small: %zu bytes needed", need); return SSO_E_ARG; }
+  return p2_prepare_devices(ops_for(p->curve), L, d, log_m, accumulator, out, devices, ndev, device, err, errcap);
+}
+
+// sso_p2_prepare_file in parts over the devices of this process.  The output (which holds the intermediate rows of the transform)
+// is created under a temporary name and renamed when the call succeeded.
+int32_t sso_p2_prepare_devices_file(const char* phase2_fn, const char* response_fn, uint64_t phase2_size, const sso_p1_params_t* p,
+                                    const int* devices, int ndev, int device, char* err, size_t errcap) {
+  if (!phase2_fn || !response_fn) { set_err(err, errcap, "null argument"); return SSO_E_ARG; }
+  P1Layout L;
+  FftDomain d;
+  int log_m;
+  int rc = p2prep_check(p, phase2_size, L, d, log_m, err, errcap, 64);
+  if (rc) return rc;
+  if ((rc = refuse_existing(phase2_fn, err, errcap))) return rc;
+  MappedFile in;
+  Outputs outs;
+  uint8_t* out;
+  if ((rc = in.open_ro(response_fn, err, errcap))) return rc;
+  if (in.len != L.acc_size) { set_err(err, errcap, "accumulator is %zu bytes, the parameters give %llu", in.len, (unsigned long long)L.acc_size); return SSO_E_ARG; }
+  if ((rc = outs.create_mapped(phase2_fn, p2prep_size(L.cs, phase2_size), true, &out, err, errcap))) return rc;
+  if ((rc = p2_prepare_devices(ops_for(p->curve), L, d, log_m, in.p, out, devices, ndev, device, err, errcap))) return rc;
+  return outs.commit(err, errcap);
+}
+
 int32_t sso_imad_peak(int device, int variant, double* macs_per_s, char* err, size_t errcap) {
   Ctx c(err, errcap);
   int rc = c.init(device);

@@ -65,6 +65,15 @@ struct CurveOps {
   // d_out[j] = d_hi[j] - d_lo[j] for n uncompressed points
   int (*points_sub)(Ctx& c, int si, uint32_t group, const uint8_t* d_hi, const uint8_t* d_lo, uint64_t n, uint8_t* d_out,
                     uint32_t out_compressed, char* err, size_t errcap);
+  // tau tables (run_tau_tables) for the part twiddle of the four-step group FFT: tau = w^e, w = root^(2^squarings) (root: host,
+  // canonical words), first index 0, coefficient slot 0 = scale (host, canonical Fr bytes; null = 1)
+  int (*fft_part_tables)(Ctx& c, int si, const uint32_t* root, uint32_t squarings, uint64_t e, const uint8_t* scale, uint32_t** d_table,
+                         char* err, size_t errcap);
+  // Stockham stage log_ns of the FFT over `rows` rows of row_len uncompressed points (a power of two), natural order in and out:
+  // the upper half times w^(row mod 2^log_ns) (w: root^(2^(two_adicity - log_ns - 1)), as in group_fft), then the row butterflies
+  // (kernels.cuh body_fft_row_butterfly): d_x -> d_out
+  int (*fft_row_stage)(Ctx& c, int si, uint32_t group, const uint8_t* d_x, uint64_t rows, uint64_t row_len, uint32_t log_ns, const uint32_t* root,
+                       uint32_t two_adicity, uint32_t* d_status, uint8_t* d_out, char* err, size_t errcap);
 };
 
 template <class Fr>
@@ -636,6 +645,106 @@ inline int run_group_fft(Ctx& c, int si, const uint8_t* d_x, uint32_t log_n, con
   return SSO_OK;
 }
 
+// the input of k_tau_tables for the part twiddle of the four-step group FFT: tau = w^e with w = root^(2^squarings), then the
+// coefficient slots scale (canonical; null = 1), 1, 1
+template <class Fr>
+__global__ void __launch_bounds__(128, 1) k_fft_part_root(const uint32_t* root_canon, uint32_t squarings, uint64_t e, const uint32_t* scale_canon,
+                                                        uint32_t* out_canon) {
+  if (blockIdx.x != 0 || threadIdx.x != 0) return;
+  typename Fr::T w = Fr::to_mont(Fr::from_const(root_canon));
+  for (uint32_t i = 0; i < squarings; i++) w = Fr::sqr(w);
+  w = Fr::from_mont(fr_pow_u64<Fr>(w, e));
+  for (int i = 0; i < Fr::L; i++) out_canon[i] = w.v[i];
+  for (int k = 1; k <= TAU_COEFF_SLOTS; k++)
+    for (int i = 0; i < Fr::L; i++) out_canon[k * Fr::L + i] = k == 1 && scale_canon ? scale_canon[i] : (i == 0 ? 1u : 0u);
+}
+// t_e = w^((e >> row_shift) & tw_mask) x[e]: the twiddles of the FFT over rows of 2^row_shift points (the row index as exponent)
+template <class G>
+__global__ void __launch_bounds__(128, (G::GROUP == 0 ? SSO_EXP_MIN_BLOCKS_G1 : SSO_EXP_MIN_BLOCKS_G2)) k_fft_row_twiddle(const __grid_constant__ VecBatch batch,
+                                                    const uint32_t* table, uint32_t tw_mask, uint32_t row_shift, uint32_t* jac_out, uint32_t* status) {
+  extern __shared__ __align__(16) unsigned char tree_raw[];
+  block_batch_exp<G, true>(blockIdx.x, batch, 0, table, CHECK_NO, jac_out, status, reinterpret_cast<typename G::F::T*>(tree_raw), tw_mask, row_shift);
+}
+template <class G>
+__global__ void __launch_bounds__(128, 1) k_fft_row_butterfly(uint32_t half, uint32_t row_len, uint32_t log_ns, const uint8_t* x, const uint32_t* tw,
+                                                            uint32_t* jac_out) {
+  body_fft_row_butterfly<G>(blockIdx.x * blockDim.x + threadIdx.x, half, row_len, log_ns, x, tw, jac_out);
+}
+
+template <class Fr>
+inline int run_fft_part_tables(Ctx& c, int si, const uint32_t* root, uint32_t squarings, uint64_t e, const uint8_t* scale, uint32_t** d_table,
+                               char* err, size_t errcap) {
+  uint32_t *d_root, *d_scale = nullptr, *d_sc;
+  int rc;
+  if ((rc = upload_scalar(c, (const uint8_t*)root, (size_t)Fr::L * 4, Fr::L, &d_root, si, err, errcap))) return rc;
+  if (scale && (rc = upload_scalar(c, scale, Fr::NBYTES, Fr::L, &d_scale, si, err, errcap))) return rc;
+  if ((rc = c.alloc((void**)&d_sc, (size_t)(1 + TAU_COEFF_SLOTS) * Fr::L * 4, si))) return rc;
+  if ((rc = c.alloc((void**)d_table, (size_t)TAU_TABLE_ELEMS * Fr::L * 4, si))) return rc;
+  c.begin(PK_TAU_TABLES, si, TAU_TABLE_ELEMS);
+  k_fft_part_root<Fr><<<1, 32, 0, c.s[si]>>>(d_root, squarings, e, d_scale, d_sc);
+  k_tau_tables<Fr><<<div_up(TAU_TABLE_ELEMS, 128), 128, 0, c.s[si]>>>(d_sc, d_sc + Fr::L, 0, *d_table);
+  c.end(si);
+  CUDA_TRY(cudaGetLastError());
+  return SSO_OK;
+}
+
+// Stage log_ns of the FFT over `rows` rows of row_len points (a power of two): the twiddles of the upper half (one launch, the row
+// index as exponent of the stage root), then the row butterflies into Jacobian scratch and their normalisation into d_out
+template <class G>
+inline int run_fft_row_stage(Ctx& c, int si, const uint8_t* d_x, uint64_t rows, uint64_t row_len, uint32_t log_ns, const uint32_t* root,
+                             uint32_t two_adicity, uint32_t* d_status, uint8_t* d_out, char* err, size_t errcap) {
+  using F = typename G::F;
+  using Fr = typename G::Fr;
+  using C = SW<G>;
+  const uint64_t n = rows * row_len, half = n / 2;
+  if (rows < 2 || n > (1ull << 24) || (row_len & (row_len - 1))) {
+    set_err(err, errcap, "row FFT stage of %llu x %llu points", (unsigned long long)rows, (unsigned long long)row_len);
+    return SSO_E_ARG;
+  }
+  cudaStream_t st = c.s[si];
+  uint32_t *d_jac, *d_tw = nullptr;
+  int rc;
+  if ((rc = c.alloc((void**)&d_jac, n * 3 * F::WORDS * 4, si))) return rc;
+  if (log_ns > 0) {
+    uint32_t *d_root, *d_stage, *d_table;
+    if ((rc = upload_scalar(c, (const uint8_t*)root, (size_t)Fr::L * 4, Fr::L, &d_root, si, err, errcap))) return rc;
+    if ((rc = c.alloc((void**)&d_stage, (size_t)(1 + TAU_COEFF_SLOTS) * Fr::L * 4, si))) return rc;
+    if ((rc = c.alloc((void**)&d_table, (size_t)TAU_TABLE_ELEMS * Fr::L * 4, si))) return rc;
+    if ((rc = c.alloc((void**)&d_tw, half * 3 * F::WORDS * 4, si))) return rc;
+    c.begin(PK_OTHER, si, TAU_TABLE_ELEMS);
+    k_fft_stage_root<Fr><<<1, 32, 0, st>>>(d_root, two_adicity - (log_ns + 1), d_stage);
+    k_tau_tables<Fr><<<div_up(TAU_TABLE_ELEMS, 128), 128, 0, st>>>(d_stage, d_stage + Fr::L, 0, d_table);
+    c.end(si);
+    VecBatch b;
+    memset(&b, 0, sizeof b);
+    b.seg[0].in = d_x + half * C::SIZE_U; b.seg[0].n = (uint32_t)half; b.nseg = 1; b.total = (uint32_t)half;
+    const uint32_t mask = (1u << log_ns) - 1, shift = (uint32_t)__builtin_ctzll(row_len);
+    c.begin(G::GROUP == 0 ? PK_BATCH_EXP_G1 : PK_BATCH_EXP_G2, si, half);
+    using GC = typename CoopOf<G>::type;
+    bool coop = false;
+    if constexpr (!std::is_void<GC>::value) {
+      if (coop_g2_enabled<GC>()) {
+        coop = true;
+        if (ExpBlock<GC>::SMEM > 48 * 1024)
+          CUDA_TRY(cudaFuncSetAttribute(k_fft_row_twiddle<GC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ExpBlock<GC>::SMEM));
+        k_fft_row_twiddle<GC><<<div_up(half, ExpBlock<GC>::PPB), EXP_BLOCK, ExpBlock<GC>::SMEM, st>>>(b, d_table, mask, shift, d_tw, d_status);
+      }
+    }
+    if (!coop) {
+      constexpr size_t TREE_BYTES = 16 + 2 * EXP_BLOCK * sizeof(typename F::T);
+      if (TREE_BYTES > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(k_fft_row_twiddle<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TREE_BYTES));
+      k_fft_row_twiddle<G><<<div_up(half, EXP_BLOCK), EXP_BLOCK, TREE_BYTES, st>>>(b, d_table, mask, shift, d_tw, d_status);
+    }
+    c.end(si);
+  }
+  c.begin(PK_OTHER, si, n);
+  k_fft_row_butterfly<G><<<div_up(half, 128), 128, 0, st>>>((uint32_t)half, (uint32_t)row_len, log_ns, d_x, d_tw, d_jac);
+  c.end(si);
+  run_normalize_other<G>(c, si, d_jac, n, d_out, 0);
+  CUDA_TRY(cudaGetLastError());
+  return SSO_OK;
+}
+
 template <class G>
 inline int run_points_sub(Ctx& c, int si, const uint8_t* d_hi, const uint8_t* d_lo, uint64_t n, uint8_t* d_out, uint32_t out_compressed,
                           char* err, size_t errcap) {
@@ -737,8 +846,19 @@ template <class G1, class G2, class PP> struct CurveImpl {
     set_err(err, errcap, "unknown group %u", group);
     return SSO_E_ARG;
   }
+  static int fft_part_tables(Ctx& c, int si, const uint32_t* root, uint32_t squarings, uint64_t e, const uint8_t* scale, uint32_t** d_table,
+                             char* err, size_t errcap) {
+    return run_fft_part_tables<typename G1::Fr>(c, si, root, squarings, e, scale, d_table, err, errcap);
+  }
+  static int fft_row_stage(Ctx& c, int si, uint32_t group, const uint8_t* d_x, uint64_t rows, uint64_t row_len, uint32_t log_ns, const uint32_t* root,
+                           uint32_t two_adicity, uint32_t* d_status, uint8_t* d_out, char* err, size_t errcap) {
+    if (group == GROUP_G1) return run_fft_row_stage<G1>(c, si, d_x, rows, row_len, log_ns, root, two_adicity, d_status, d_out, err, errcap);
+    if (group == GROUP_G2) return run_fft_row_stage<G2>(c, si, d_x, rows, row_len, log_ns, root, two_adicity, d_status, d_out, err, errcap);
+    set_err(err, errcap, "unknown group %u", group);
+    return SSO_E_ARG;
+  }
   static const CurveOps* ops() {
-    static const CurveOps o = {&tau_tables, &batch_exp, &batch_exp_chunk, &reencode, &msm_pairs, &same_ratio, (uint32_t)Pairing<G1, G2, PP>::CHECK_BYTES, &keygen_g1, &keygen_scalars, &hash_to_g2, (uint32_t)G1::Fr::L, &points_sum, &fill_generator, (uint32_t)G1::Fr::NBYTES, {2u * G1::F::WORDS, 2u * G2::F::WORDS}, G2::VERIFY_WEIGHT, &group_fft, &points_sub};
+    static const CurveOps o = {&tau_tables, &batch_exp, &batch_exp_chunk, &reencode, &msm_pairs, &same_ratio, (uint32_t)Pairing<G1, G2, PP>::CHECK_BYTES, &keygen_g1, &keygen_scalars, &hash_to_g2, (uint32_t)G1::Fr::L, &points_sum, &fill_generator, (uint32_t)G1::Fr::NBYTES, {2u * G1::F::WORDS, 2u * G2::F::WORDS}, G2::VERIFY_WEIGHT, &group_fft, &points_sub, &fft_part_tables, &fft_row_stage};
     return &o;
   }
 };

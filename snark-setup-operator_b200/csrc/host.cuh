@@ -177,6 +177,12 @@ struct Ctx {
     staging.clear();
     return SSO_OK;
   }
+  // stream-ordered release of the scratch allocated since allocs.size() was `from`: a long piece hands back what one of its
+  // steps needed before the next step allocates (the pool reuses it)
+  void release(size_t from) {
+    for (size_t i = from; i < allocs.size(); i++) cudaFreeAsync(allocs[i], s[0]);
+    allocs.resize(from);
+  }
   // make stream `to` wait for everything enqueued so far on stream `from`
   int fork(int from, int to) {
     cudaEvent_t ev;

@@ -162,12 +162,12 @@ template <class G> struct ExpTypes {
 };
 
 // staged_src: the thread's serialized input point in shared memory (block_stage_input), or null = read it from global memory
-// TWIDDLE (group FFT, body_fft_butterfly): the scalar of element j is tau^(j & tw_mask) — the table holds the powers of the
+// TWIDDLE (group FFT, body_fft_butterfly): the scalar of element j is tau^((j >> tw_shift) & tw_mask) — the table holds the powers of the
 // stage's root of unity, so each butterfly gets its twiddle without a pow per point; the segment's scalar rule is not read
 template <class G, bool TWIDDLE = false>
 __device__ __forceinline__ typename G::F::T exp_stage_a(uint32_t tid, const VecBatch& b, uint32_t in_compressed, const uint32_t* table,
                                                         uint32_t check, uint32_t* status, typename ExpTypes<G>::State& st,
-                                                        const uint8_t* staged_src = nullptr, uint32_t tw_mask = 0) {
+                                                        const uint8_t* staged_src = nullptr, uint32_t tw_mask = 0, uint32_t tw_shift = 0) {
   using C = SW<G>;
   using F = typename G::F;
   using Fr = typename G::Fr;
@@ -189,7 +189,7 @@ __device__ __forceinline__ typename G::F::T exp_stage_a(uint32_t tid, const VecB
   }
   uint32_t k[Fr::L];
   if constexpr (TWIDDLE) {
-    scalar_for_index<Fr>(table, j & tw_mask, tw_mask + 1, false, 0, k);
+    scalar_for_index<Fr>(table, (j >> tw_shift) & tw_mask, tw_mask + 1, false, 0, k);
   } else if (sg.mode == 0) {
     scalar_for_index<Fr>(table, j, sg.n, sg.has_coeff != 0, sg.coeff_slot, k);
   } else {
@@ -294,7 +294,8 @@ template <class G> struct ExpBlock {
 // Cooperative body (coop.cuh): DEG lanes per point.  The tree holds one array of 2 PPB coefficients per role.
 template <class G, bool TWIDDLE = false>
 __device__ __forceinline__ void block_batch_exp_coop(uint32_t block, const VecBatch& b, const uint32_t* table, uint32_t check,
-                                                     uint32_t* jac_out, uint32_t* status, unsigned char* smem, uint32_t tw_mask = 0) {
+                                                     uint32_t* jac_out, uint32_t* status, unsigned char* smem, uint32_t tw_mask = 0,
+                                                     uint32_t tw_shift = 0) {
   using F = typename G::F;
   using CO = Coop<F::DEG>;
   constexpr int PPB = ExpBlock<G>::PPB, TL = ExpBlock<G>::TL;
@@ -303,7 +304,7 @@ __device__ __forceinline__ void block_batch_exp_coop(uint32_t block, const VecBa
   const uint32_t pb = lane_ok ? CO::group_in_block() : 0xffffffffu;
   const uint32_t tid = lane_ok ? block * PPB + pb : 0xffffffffu;       // idle lanes locate nothing and never exchange
   const uint8_t* staged = block_stage_input<G, PPB>(block, b, 0, smem, pb);
-  typename F::T leaf = exp_stage_a<G, TWIDDLE>(tid, b, 0, table, check, status, st, staged, tw_mask);
+  typename F::T leaf = exp_stage_a<G, TWIDDLE>(tid, b, 0, table, check, status, st, staged, tw_mask, tw_shift);
   __syncthreads();
   if constexpr (G::AFFINE_TABLE) {
     typename F::T* tree = reinterpret_cast<typename F::T*>(smem) + (size_t)(lane_ok ? CO::role() : 0) * 2 * TL;
@@ -325,14 +326,14 @@ __device__ __forceinline__ void block_batch_exp_coop(uint32_t block, const VecBa
 template <class G, bool TWIDDLE = false>
 __device__ __forceinline__ void block_batch_exp(uint32_t block, const VecBatch& b, uint32_t in_compressed, const uint32_t* table,
                                                 uint32_t check, uint32_t* jac_out, uint32_t* status, typename G::F::T* tree,
-                                                uint32_t tw_mask = 0) {
+                                                uint32_t tw_mask = 0, uint32_t tw_shift = 0) {
   if constexpr (G::F::COOP != 0) {
-    block_batch_exp_coop<G, TWIDDLE>(block, b, table, check, jac_out, status, reinterpret_cast<unsigned char*>(tree), tw_mask);
+    block_batch_exp_coop<G, TWIDDLE>(block, b, table, check, jac_out, status, reinterpret_cast<unsigned char*>(tree), tw_mask, tw_shift);
   } else {
     typename ExpTypes<G>::State st;
     uint32_t tid = block * EXP_BLOCK + threadIdx.x;
     const uint8_t* staged = block_stage_input<G>(block, b, in_compressed, reinterpret_cast<uint8_t*>(tree));
-    typename G::F::T leaf = exp_stage_a<G, TWIDDLE>(tid, b, in_compressed, table, check, status, st, staged, tw_mask);
+    typename G::F::T leaf = exp_stage_a<G, TWIDDLE>(tid, b, in_compressed, table, check, status, st, staged, tw_mask, tw_shift);
     __syncthreads();                                                  // the staged bytes are dead: the tree may take the buffer
     if constexpr (G::AFFINE_TABLE) {
       tree[EXP_BLOCK + threadIdx.x] = leaf;
@@ -473,6 +474,42 @@ __device__ __forceinline__ void body_fft_butterfly(uint32_t j, uint32_t half, ui
   F::store(base + (size_t)F::WORDS * n, n, s.Y);
   F::store(base + (size_t)2 * F::WORDS * n, n, s.Z);
   base += ns;
+  F::store(base, n, d.X);
+  F::store(base + (size_t)F::WORDS * n, n, d.Y);
+  F::store(base + (size_t)2 * F::WORDS * n, n, d.Z);
+}
+
+// The cross-part FFT of the four-step group FFT (p2prep.cuh): the stage above over rows of row_len points instead of single points.
+// x holds 2 half points (uncompressed), row r at [r row_len, (r + 1) row_len).  For e < half, row j = e / row_len, column col:
+//   a = x[e],  t = w^(j mod Ns) x[e + half] (tw: the twiddle batch_exp over the upper half with the row index as exponent, Jacobian SoA;
+//   null in stage 0, whose twiddle is 1);  a + t to row o = 2 Ns floor(j / Ns) + (j mod Ns), a - t to row o + Ns, column col.
+template <class G>
+__device__ __forceinline__ void body_fft_row_butterfly(uint32_t e, uint32_t half, uint32_t row_len, uint32_t log_ns, const uint8_t* x,
+                                                       const uint32_t* tw, uint32_t* jac_out) {
+  using C = SW<G>;
+  using F = typename G::F;
+  if (e >= half) return;
+  const uint32_t j = e / row_len, col = e - j * row_len;
+  typename C::Affine pa, pb;
+  C::read_uncompressed(x + (size_t)e * C::SIZE_U, pa);
+  typename C::Jac a = C::from_affine(pa), t;
+  if (tw) {
+    t.X = F::load(tw + e, half);
+    t.Y = F::load(tw + (size_t)F::WORDS * half + e, half);
+    t.Z = F::load(tw + (size_t)2 * F::WORDS * half + e, half);
+  } else {
+    C::read_uncompressed(x + ((size_t)e + half) * C::SIZE_U, pb);
+    t = C::from_affine(pb);
+  }
+  const typename C::Jac s = C::add(a, t), d = C::add(a, C::neg(t));
+  const uint32_t ns = 1u << log_ns;
+  const uint32_t o = ((j >> log_ns) << (log_ns + 1)) + (j & (ns - 1));
+  const size_t n = (size_t)2 * half;
+  uint32_t* base = jac_out + (size_t)o * row_len + col;
+  F::store(base, n, s.X);
+  F::store(base + (size_t)F::WORDS * n, n, s.Y);
+  F::store(base + (size_t)2 * F::WORDS * n, n, s.Z);
+  base += (size_t)ns * row_len;
   F::store(base, n, d.X);
   F::store(base + (size_t)F::WORDS * n, n, d.Y);
   F::store(base + (size_t)2 * F::WORDS * n, n, d.Z);

@@ -92,26 +92,59 @@ def group_fft(curve, group: int, d_in, log_n: int, d_out, inverse=False, in_comp
          int(out_compressed), device)
 
 
-def prepare_phase2_buf(parameters, accumulator, phase2_size: int, device=0) -> bytes:
+def _devices(devices, device):
+    """devices=None: (no list, `device`); -1: every visible device; a list: those devices (an entry may repeat: one more worker)."""
+    from .phase1 import _devices_arg
+    if devices == -1:
+        return None, 0, -1
+    arr, n = _devices_arg(list(devices))
+    return arr, n, device
+
+
+def group_fft_parts(curve, group: int, data, log_n: int, parts: int, inverse=False, devices=None, device=0) -> bytes:
+    """The transform of group_fft on host bytes (2^log_n uncompressed points) as a four-step FFT in `parts` parts (a power of two,
+    2^log_n / parts <= 2^24), spread over `devices` (None: `device`; -1: all visible; a list may repeat a device)."""
+    from .phase1 import _host_ptr
+    s = curve_sizes(curve)
+    ptr, n, keep = _host_ptr(data)
+    out = ctypes.create_string_buffer((1 << log_n) * (s["g1_u"] if group == 0 else s["g2_u"]))
+    arr, nd, dev = _devices([] if devices is None else devices, device)
+    call("sso_group_fft_parts_buf", curve_id(curve), group, ptr, n, log_n, int(inverse), out, len(out), parts, arr, nd, dev)
+    del keep
+    return out.raw
+
+
+def prepare_phase2_buf(parameters, accumulator, phase2_size: int, device=0, devices=None) -> bytes:
     """phase2_cli::prepare_phase2 on host buffers: a Full-mode accumulator (uncompressed, `parameters` a Phase1Parameters) ->
     the Lagrange-basis Groth16Params of phase2_size points (alpha_g1 | beta_g1 | beta_g2 | coeffs_g1 | coeffs_g2 |
-    alpha_coeffs_g1 | beta_coeffs_g1 | h_g1, uncompressed)."""
+    alpha_coeffs_g1 | beta_coeffs_g1 | h_g1, uncompressed).  devices=None: the transform in one piece on `device` (at most 2^24
+    points); a list of devices (an entry may repeat: one more worker) or -1 (all visible): the transform in parts, the same bytes,
+    up to the radix-2 domain of the curve."""
     from ._lib import SsoError, lib
     from .phase1 import _host_ptr
     ptr, n, keep = _host_ptr(accumulator)
     need = ctypes.c_size_t(0)
     err = ctypes.create_string_buffer(512)
     p = parameters.c_struct()
-    rc = lib().sso_p2_prepare_buf(ctypes.byref(p), ptr, n, phase2_size, None, 0, ctypes.byref(need), device, err, len(err))
+    if devices is None:
+        fn, tail = "sso_p2_prepare_buf", (device,)
+    else:
+        fn, tail = "sso_p2_prepare_devices_buf", _devices(devices, device)
+    rc = getattr(lib(), fn)(ctypes.byref(p), ptr, n, phase2_size, None, 0, ctypes.byref(need), *tail, err, len(err))
     if rc != -1 or need.value == 0:
         raise SsoError(rc, err.value.decode("utf-8", "replace"))
     out = ctypes.create_string_buffer(need.value)
-    call("sso_p2_prepare_buf", ctypes.byref(p), ptr, n, phase2_size, out, len(out), ctypes.byref(need), device)
+    call(fn, ctypes.byref(p), ptr, n, phase2_size, out, len(out), ctypes.byref(need), *tail)
     del keep
     return out.raw
 
 
-def prepare_phase2(phase2_filename, response_filename, phase2_size: int, parameters, device=0):
-    """phase2_cli::prepare_phase2, argument for argument (reference src/bin/intermediate_transform.rs:213-226)."""
-    call("sso_p2_prepare_file", phase2_filename.encode(), response_filename.encode(), phase2_size, ctypes.byref(parameters.c_struct()),
-         device)
+def prepare_phase2(phase2_filename, response_filename, phase2_size: int, parameters, device=0, devices=None):
+    """phase2_cli::prepare_phase2, argument for argument (reference src/bin/intermediate_transform.rs:213-226).  devices as for
+    prepare_phase2_buf."""
+    if devices is None:
+        call("sso_p2_prepare_file", phase2_filename.encode(), response_filename.encode(), phase2_size, ctypes.byref(parameters.c_struct()),
+             device)
+        return
+    call("sso_p2_prepare_devices_file", phase2_filename.encode(), response_filename.encode(), phase2_size,
+         ctypes.byref(parameters.c_struct()), *_devices(devices, device))
