@@ -348,7 +348,7 @@ int32_t sso_p2_prepare_file(const char* phase2_fn, const char* response_fn, uint
 /* The same transforms in parts: a four-step group FFT (2^log_n = parts * M points; per part a size-M FFT of the stride-`parts`
  * subsequence and its twiddles, then per block of columns a `parts`-point FFT over the rows), with the output buffer (or file) as the
  * exchange buffer and device memory per task of the order of one part.  They run on the devices of the calling process, never
- * cooperatively over a process group: devices[0..ndev) (NULL / 0: `device`; device = -1: all visible); an entry may repeat, for one
+ * cooperatively over a process group (that is sso_p2_prepare_dist_file): devices[0..ndev) (NULL / 0: `device`; device = -1: all visible); an entry may repeat, for one
  * more worker on that device.  Every size and argument check comes before any device use.
  *
  * Group FFT of 2^log_n uncompressed points on HOST buffers in `parts` parts (a power of two up to 2^24, 2^log_n / parts <= 2^24; log_n up to the
@@ -365,6 +365,17 @@ int32_t sso_p2_prepare_devices_buf(const sso_p1_params_t* p, const uint8_t* accu
                                    size_t out_cap, size_t* out_len, const int* devices, int ndev, int device, char* err, size_t errcap);
 int32_t sso_p2_prepare_devices_file(const char* phase2_fn, const char* response_fn, uint64_t phase2_size, const sso_p1_params_t* p,
                                     const int* devices, int ndev, int device, char* err, size_t errcap);
+/* sso_p2_prepare_devices_file as a cooperative call of the process group (sso_dist_init): every rank calls it with the same
+ * arguments, computes its share of the parts and of h_g1 on its own GPU (the `device` of sso_dist_init) and writes it into the
+ * shared mapping of the output; the output bytes are those of sso_p2_prepare_buf for any world size and number of parts.
+ * parts = 0 chooses the number of parts as sso_p2_prepare_devices_file does, with one worker per rank and the least free device
+ * memory of any rank; otherwise a power of two up to phase2_size, with parts of at most 2^24 points.  Without a process group:
+ * SSO_E_ARG before any device use.  Arguments that differ between the ranks (parameters, phase2_size, parts, the accumulator's
+ * length or hash slot): SSO_E_ARG on every rank.  A failure on one rank (an existing output: SSO_E_IO; a rejected accumulator
+ * element) makes the call fail on every rank, and neither the output nor <phase2_fn>.sso-partial remains.  Like every cooperative
+ * call, it needs all ranks to map the same files: one host, or a file system whose shared mappings are coherent between them. */
+int32_t sso_p2_prepare_dist_file(const char* phase2_fn, const char* response_fn, uint64_t phase2_size, const sso_p1_params_t* p,
+                                 uint64_t parts, char* err, size_t errcap);
 
 /* setup_utils::calculate_hash (reference src/utils.rs:618-623): Blake2b-512, unkeyed. Host only. */
 int32_t sso_blake2b_512(const uint8_t* data, size_t len, uint8_t out[64]);

@@ -89,6 +89,7 @@ def lib() -> ctypes.CDLL:
         L.sso_group_fft_parts_buf.argtypes = [u32, u32, vp, sz, u32, u32, vp, sz, u64, ip, i32, i32, cp, sz]
         L.sso_p2_prepare_devices_buf.argtypes = [pp, vp, sz, u64, vp, sz, szp, ip, i32, i32, cp, sz]
         L.sso_p2_prepare_devices_file.argtypes = [cp, cp, u64, pp, ip, i32, i32, cp, sz]
+        L.sso_p2_prepare_dist_file.argtypes = [cp, cp, u64, pp, u64, cp, sz]
         L.sso_profile_enable.argtypes = [ctypes.c_int32]
         L.sso_profile_read.argtypes = [ctypes.POINTER(u64), sz]
         L.sso_imad_peak.argtypes = [i32, i32, ctypes.POINTER(ctypes.c_double), cp, sz]
@@ -104,7 +105,7 @@ def lib() -> ctypes.CDLL:
                      "sso_p2_contribute_buf", "sso_p2_contribute_file", "sso_p2_verify_buf", "sso_p2_verify_file",
                      "sso_dist_unique_id", "sso_dist_init", "sso_dist_barrier", "sso_dist_finalize", "sso_dist_stats", "sso_p1_contribute_seeded_many_buf",
                      "sso_group_fft_dev", "sso_p2_prepare_buf", "sso_p2_prepare_file", "sso_group_fft_parts_buf",
-                     "sso_p2_prepare_devices_buf", "sso_p2_prepare_devices_file"):
+                     "sso_p2_prepare_devices_buf", "sso_p2_prepare_devices_file", "sso_p2_prepare_dist_file"):
             getattr(L, name).restype = ctypes.c_int32
         _lib = L
     return _lib

@@ -1505,7 +1505,10 @@ int32_t sso_p2_prepare_devices_buf(const sso_p1_params_t* p, const uint8_t* accu
   const size_t need = p2prep_size(L.cs, phase2_size);
   *out_len = need;
   if (!out || out_cap < need) { set_err(err, errcap, "output buffer too small: %zu bytes needed", need); return SSO_E_ARG; }
-  return p2_prepare_devices(ops_for(p->curve), L, d, log_m, accumulator, out, devices, ndev, device, err, errcap);
+  Participants Pt;
+  uint32_t log_p;
+  if ((rc = p2_local_plan(L.cs, log_m, devices, ndev, device, Pt, log_p, err, errcap))) return rc;
+  return p2_prepare_devices(ops_for(p->curve), L, d, log_m, log_p, accumulator, out, Pt, err, errcap);
 }
 
 // sso_p2_prepare_file in parts over the devices of this process.  The output (which holds the intermediate rows of the transform)
@@ -1524,9 +1527,83 @@ int32_t sso_p2_prepare_devices_file(const char* phase2_fn, const char* response_
   uint8_t* out;
   if ((rc = in.open_ro(response_fn, err, errcap))) return rc;
   if (in.len != L.acc_size) { set_err(err, errcap, "accumulator is %zu bytes, the parameters give %llu", in.len, (unsigned long long)L.acc_size); return SSO_E_ARG; }
+  Participants Pt;
+  uint32_t log_p;
+  if ((rc = p2_local_plan(L.cs, log_m, devices, ndev, device, Pt, log_p, err, errcap))) return rc;
   if ((rc = outs.create_mapped(phase2_fn, p2prep_size(L.cs, phase2_size), true, &out, err, errcap))) return rc;
-  if ((rc = p2_prepare_devices(ops_for(p->curve), L, d, log_m, in.p, out, devices, ndev, device, err, errcap))) return rc;
+  if ((rc = p2_prepare_devices(ops_for(p->curve), L, d, log_m, log_p, in.p, out, Pt, err, errcap))) return rc;
   return outs.commit(err, errcap);
+}
+
+// sso_p2_prepare_devices_file as a cooperative call of the process group: every rank makes the same call, computes its share of
+// the parts on the device of sso_dist_init, and writes it into the shared mapping of the output.  The ranks agree after every step,
+// so that no rank waits in a collective another rank has left:
+//   1. the argument checks of sso_p2_prepare_devices_file, on every rank (the existing output and the accumulator length too);
+//   2. one min and one max all-reduce over the arguments, the accumulator's length and hash slot, every rank's failure flag and its
+//      free device memory: a difference between ranks is SSO_E_ARG on every rank, the plan (parts = 0: choose_parts over `world`
+//      workers with the least free memory of any rank) is the same on every rank;
+//   3. the output transaction of file_call: rank 0 creates <phase2_fn>.sso-partial, every rank works, rank 0 commits.
+int32_t sso_p2_prepare_dist_file(const char* phase2_fn, const char* response_fn, uint64_t phase2_size, const sso_p1_params_t* p,
+                                 uint64_t parts, char* err, size_t errcap) {
+  P1Layout L;
+  FftDomain d;
+  int log_m = 0, log_p = -1;
+  int rc = SSO_OK;
+  if (!phase2_fn || !response_fn) { set_err(err, errcap, "null argument"); rc = SSO_E_ARG; }
+  if (!rc) rc = p2prep_check(p, phase2_size, L, d, log_m, err, errcap, 64);
+  if (!rc && parts) {
+    log_p = log2_exact(parts);
+    if (log_p < 0 || log_p > log_m || log_m - log_p > 24) {
+      set_err(err, errcap, "%llu parts of 2^%d points: a power of two up to the number of points, with parts of at most 2^24 points",
+              (unsigned long long)parts, log_m);
+      rc = SSO_E_ARG;
+    }
+  }
+  // a rank with bad arguments still takes part in the agreement below when a process group exists
+  if (!dist_state().on) {
+    if (!rc) { set_err(err, errcap, "sso_p2_prepare_dist_file needs a process group (sso_dist_init)"); rc = SSO_E_ARG; }
+    return rc;
+  }
+  MappedFile in;
+  Participants Pt;
+  uint64_t avail = 0;
+  if (!rc) rc = refuse_existing(phase2_fn, err, errcap);
+  if (!rc) rc = in.open_ro(response_fn, err, errcap);
+  if (!rc && in.len != L.acc_size) {
+    set_err(err, errcap, "accumulator is %zu bytes, the parameters give %llu", in.len, (unsigned long long)L.acc_size);
+    rc = SSO_E_ARG;
+  }
+  if (!rc) rc = resolve_participants(nullptr, 0, 0, true, Pt, err, errcap);
+  if (!rc) rc = free_per_worker(Pt, avail, err, errcap);
+  // [0] failure flag | [1, 15) the fingerprint every rank must share (the last 8 words: the hash slot) | [15] free device memory
+  enum { FAILED = 0, FP_FIRST = 1, HASH = 7, FP_END = 15, AVAIL = 15, NWORDS = 16 };
+  static const char* const field[HASH] = {"", "curve", "power", "contribution mode", "phase-2 size", "parts", "accumulator length"};
+  uint64_t lo[NWORDS] = {0};
+  lo[FAILED] = rc != SSO_OK;
+  if (!rc) {
+    lo[1] = p->curve; lo[2] = p->power; lo[3] = p->contribution_mode; lo[4] = phase2_size; lo[5] = parts; lo[6] = in.len;
+    memcpy(&lo[HASH], in.p, 64);
+    lo[AVAIL] = avail;
+  }
+  uint64_t hi[NWORDS];
+  memcpy(hi, lo, sizeof lo);
+  char e2[256];
+  e2[0] = 0;
+  int32_t rc2 = dist_reduce_u64(lo, NWORDS, false, e2, sizeof e2);
+  if (!rc2) rc2 = dist_reduce_u64(hi, NWORDS, true, e2, sizeof e2);
+  if (rc) return rc;
+  if (rc2) { set_err(err, errcap, "%s", e2); return rc2; }
+  if (hi[FAILED]) { set_err(err, errcap, "another rank of the process group refused the call's arguments"); return SSO_E_ARG; }
+  for (int i = FP_FIRST; i < FP_END; i++)
+    if (lo[i] != hi[i]) {
+      set_err(err, errcap, "the ranks of the process group called with different arguments (%s)", i < HASH ? field[i] : "accumulator hash slot");
+      return SSO_E_ARG;
+    }
+  uint32_t lp = (uint32_t)log_p;
+  if (log_p < 0 && (rc = choose_parts((uint32_t)log_m, std::max(L.cs.g1u, L.cs.g2u), (uint64_t)Pt.world, lo[AVAIL], lp, err, errcap))) return rc;
+  return file_call(true, phase2_fn, p2prep_size(L.cs, phase2_size), [] { return (int32_t)SSO_OK; },
+      [&](uint8_t* out) { return p2_prepare_devices(ops_for(p->curve), L, d, log_m, lp, in.p, out, Pt, err, errcap); },
+      [](Outputs&, const uint8_t*) { return (int32_t)SSO_OK; }, err, errcap);
 }
 
 int32_t sso_imad_peak(int device, int variant, double* macs_per_s, char* err, size_t errcap) {

@@ -173,11 +173,10 @@ struct PartsVec { uint32_t group; const uint8_t* in; uint8_t* out; uint32_t vec;
 // and needs less per point
 inline uint64_t parts_footprint(uint64_t M, size_t sz) { return 7 * std::max<uint64_t>(M, 1ull << 18) * sz + (64ull << 20); }
 
-// The number of parts of prepare_phase2 in parts: the smallest power of two P <= m such that P >= the number of workers,
-// m / P <= 2^24 and a part of the widest vector (sz bytes a point) fits the free memory of its device (cudaMemGetInfo at call
-// start) divided among the workers there.
-inline int choose_parts(uint32_t log_m, size_t sz, const Participants& Pt, uint32_t& log_p, char* err, size_t errcap) {
-  uint64_t per_worker = ~0ull;
+// The free memory of a worker of Pt: the least over its devices of the free memory (cudaMemGetInfo at call start) divided among
+// the workers there
+inline int free_per_worker(const Participants& Pt, uint64_t& per_worker, char* err, size_t errcap) {
+  per_worker = ~0ull;
   int prev = 0;
   CUDA_TRY(cudaGetDevice(&prev));
   for (int dev : Pt.devices) {
@@ -188,7 +187,12 @@ inline int choose_parts(uint32_t log_m, size_t sz, const Participants& Pt, uint3
     per_worker = std::min<uint64_t>(per_worker, avail / on_dev);
   }
   CUDA_TRY(cudaSetDevice(prev));
-  const uint64_t workers = Pt.devices.size();
+  return SSO_OK;
+}
+
+// The number of parts of prepare_phase2 in parts: the smallest power of two P <= m such that P >= the number of workers,
+// m / P <= 2^24 and a part of the widest vector (sz bytes a point) fits the free memory of a worker.
+inline int choose_parts(uint32_t log_m, size_t sz, uint64_t workers, uint64_t per_worker, uint32_t& log_p, char* err, size_t errcap) {
   auto fits = [&](uint32_t lp) { return log_m - lp <= 24 && parts_footprint(1ull << (log_m - lp), sz) <= per_worker; };
   log_p = 0;
   while (log_p < log_m && ((1ull << log_p) < workers || !fits(log_p))) log_p++;
@@ -287,7 +291,9 @@ inline int parts_block(Ctx& c, const CurveOps* ops, const CurveSizes& cs, const 
 
 // Both passes over the workers of Pt (one context each; stream.cuh run_pieces: the first failure wins, no further task starts and
 // every worker is joined).  Pass 1 deals the parts vector by vector in the order given (the costlier G2 vector first), then the
-// `extra` tasks (extra_task(i, ...)); pass 2 the column blocks.
+// `extra` tasks (extra_task(i, ...)); pass 2 the column blocks.  In a cooperative call (Pt.dist) the tasks are dealt over the
+// ranks too, and the ranks agree after pass 1: pass 2 reads rows that other ranks wrote, and a rank whose part failed its check
+// stops every rank before pass 2.
 inline int parts_fft(const CurveOps* ops, const CurveSizes& cs, const PartsPlan& pl, const PartsVec* vecs, size_t nvec, const Participants& Pt,
                      uint32_t check, const char* what, size_t extra, const std::function<int(size_t, Ctx&, char*, size_t)>& extra_task,
                      char* err, size_t errcap) {
@@ -295,6 +301,7 @@ inline int parts_fft(const CurveOps* ops, const CurveSizes& cs, const PartsPlan&
     if (i >= nvec * pl.P) return extra_task(i - nvec * pl.P, c, e, ec);
     return parts_part(c, ops, cs, pl, vecs[i / pl.P], i % pl.P, check, what, e, ec);
   });
+  rc = agree(Pt, rc, err, errcap);
   if (rc || pl.P == 1) return rc;
   const uint64_t nb = pl.M / pl.B;
   return run_pieces(nvec * nb, Pt, 1, 1, err, errcap, [&](size_t i, int, Ctx& c, char* e, size_t ec) -> int {
@@ -302,18 +309,23 @@ inline int parts_fft(const CurveOps* ops, const CurveSizes& cs, const PartsPlan&
   });
 }
 
-// prepare_phase2 in parts over the devices of this process (not cooperative over a process group): the four coefficient vectors by
-// parts_fft, h_g1 in pieces of at most M (its upper inputs tauG1[m .. 2m - 1) checked there; the lower ones are the parts of tauG1),
-// and the three single elements checked and re-encoded as in the transform in one piece
-inline int p2_prepare_devices(const CurveOps* ops, const P1Layout& L, const FftDomain& d, int log_m, const uint8_t* acc, uint8_t* out,
-                              const int* devices, int ndev, int device, char* err, size_t errcap) {
-  Participants Pt;
+// The workers and the number of parts of prepare_phase2 in parts over the devices of this process
+inline int p2_local_plan(const CurveSizes& cs, int log_m, const int* devices, int ndev, int device, Participants& Pt, uint32_t& log_p,
+                         char* err, size_t errcap) {
+  uint64_t per_worker;
   int rc = resolve_participants(devices, ndev, device, false, Pt, err, errcap);
   if (rc) return rc;
+  if ((rc = free_per_worker(Pt, per_worker, err, errcap))) return rc;
+  return choose_parts((uint32_t)log_m, std::max(cs.g1u, cs.g2u), Pt.devices.size(), per_worker, log_p, err, errcap);
+}
+
+// prepare_phase2 in 2^log_p parts over the workers of Pt (the devices of this process, or a cooperative call of the process group):
+// the four coefficient vectors by parts_fft, h_g1 in pieces of at most M (its upper inputs tauG1[m .. 2m - 1) checked there; the
+// lower ones are the parts of tauG1), and the three single elements checked and re-encoded as in the transform in one piece
+inline int p2_prepare_devices(const CurveOps* ops, const P1Layout& L, const FftDomain& d, int log_m, uint32_t log_p, const uint8_t* acc,
+                              uint8_t* out, const Participants& Pt, char* err, size_t errcap) {
   const CurveSizes& cs = L.cs;
   const uint64_t m = 1ull << log_m;
-  uint32_t log_p;
-  if ((rc = choose_parts((uint32_t)log_m, std::max(cs.g1u, cs.g2u), Pt, log_p, err, errcap))) return rc;
   const std::vector<uint8_t> minv = fft_inv_size(d, (uint32_t)log_m, ops->fr_bytes);
   const PartsPlan pl = parts_plan((uint32_t)log_m, log_p, d.root_inv, d.two_adicity, minv.data());
   const size_t g1 = cs.g1u, g2 = cs.g2u;

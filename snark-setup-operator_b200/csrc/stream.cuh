@@ -193,6 +193,28 @@ inline int32_t dist_sum(int32_t mine, int32_t* total, char* err, size_t errcap) 
   return SSO_OK;
 }
 
+// all-reduce (min, or max when `take_max`) of n 64-bit words across the group, in place: how the ranks of a cooperative call
+// compare their arguments and agree on a plan.  No all-gather: sso_dist_stats does not count it.
+inline int32_t dist_reduce_u64(uint64_t* v, size_t n, bool take_max, char* err, size_t errcap) {
+  DistState& d = dist_state();
+  if (!d.on || d.world == 1 || n == 0) return SSO_OK;
+  const NcclApi* api = nccl_api(err, errcap);
+  if (!api) return SSO_E_CUDA;
+  Ctx c(err, errcap);
+  int rc = c.init(d.device);
+  if (rc) return rc;
+  uint64_t* d_v;
+  if ((rc = c.alloc((void**)&d_v, n * 8))) return rc;
+  CUDA_TRY(cudaMemcpyAsync(d_v, v, n * 8, cudaMemcpyHostToDevice, c.s[0]));
+  {
+    std::lock_guard<std::mutex> g(dist_mutex());
+    NCCL_TRY(api, api->AllReduce(d_v, d_v, n, ncclUint64, take_max ? ncclMax : ncclMin, d.comm, c.s[0]));
+  }
+  CUDA_TRY(cudaMemcpyAsync(v, d_v, n * 8, cudaMemcpyDeviceToHost, c.s[0]));
+  CUDA_TRY(cudaStreamSynchronize(c.s[0]));
+  return SSO_OK;
+}
+
 // Every rank of a cooperative call must take the same path through the collectives: after a phase that can fail on one
 // rank only (a bad element sits in ONE rank's piece), the failure flags are summed and every rank leaves together.
 inline int32_t agree(const Participants& P, int32_t rc, char* err, size_t errcap) {

@@ -139,9 +139,20 @@ def prepare_phase2_buf(parameters, accumulator, phase2_size: int, device=0, devi
     return out.raw
 
 
-def prepare_phase2(phase2_filename, response_filename, phase2_size: int, parameters, device=0, devices=None):
+def prepare_phase2(phase2_filename, response_filename, phase2_size: int, parameters, device=0, devices=None, group=False, parts=0):
     """phase2_cli::prepare_phase2, argument for argument (reference src/bin/intermediate_transform.rs:213-226).  devices as for
-    prepare_phase2_buf."""
+    prepare_phase2_buf.  group=True: a cooperative call of the process group (dist_init_from_torch): every rank makes the same call on the
+    same files and computes its share of the transform in parts on its own GPU; `parts` (a power of two; 0: chosen automatically)
+    is the number of parts.  All ranks must map the same files: one host, or a file system whose shared mappings are coherent
+    between them."""
+    if group:
+        if devices is not None:
+            raise ValueError("group=True runs on the device of each rank; devices does not apply")
+        call("sso_p2_prepare_dist_file", phase2_filename.encode(), response_filename.encode(), phase2_size,
+             ctypes.byref(parameters.c_struct()), parts)
+        return
+    if parts:
+        raise ValueError("parts applies to group=True")
     if devices is None:
         call("sso_p2_prepare_file", phase2_filename.encode(), response_filename.encode(), phase2_size, ctypes.byref(parameters.c_struct()),
              device)
