@@ -134,8 +134,10 @@ __global__ void __launch_bounds__(128, 1) k_reencode(uint32_t n, const uint8_t* 
 // Both groups of a chunk in ONE launch: blocks [0, nb2) take G2 points (the long-running ones, scheduled first),
 // the rest take G1 points.  All blocks have the same register footprint, so G1 blocks fill the SMs that the last,
 // partial wave of G2 blocks leaves idle (two separate launches lose ~13 % each to wave quantisation).
+// Two resident blocks per SM: the one-thread BLS12-377 G2 body takes all 255 registers (2 x 128 threads x 255 fill the register
+// file); three blocks cap it at 168 registers and it spills (measured slower, DESIGN.md §4).
 #ifndef SSO_CHUNK_MIN_BLOCKS
-#define SSO_CHUNK_MIN_BLOCKS 1
+#define SSO_CHUNK_MIN_BLOCKS 2
 #endif
 template <class G1, class G2>
 __global__ void __launch_bounds__(128, SSO_CHUNK_MIN_BLOCKS) k_batch_exp_chunk(const __grid_constant__ VecBatch b1, const __grid_constant__ VecBatch b2,
@@ -148,6 +150,16 @@ __global__ void __launch_bounds__(128, SSO_CHUNK_MIN_BLOCKS) k_batch_exp_chunk(c
   } else {
     block_batch_exp<G1>(blockIdx.x - nb2, b1, in_compressed, table, check, jac1, status, reinterpret_cast<typename G1::F::T*>(tree_raw));
   }
+}
+// The G1 blocks of a chunk that the fused launch does not need for filling the slots its last G2 wave leaves: a G1-only kernel at
+// three resident blocks per SM (the 12-limb G1 body fits 168 registers; the fused launch runs everything at the 255 of the G2 body),
+// on a second stream beside the fused launch, so that its blocks take the slots the fused launch frees while its last blocks run
+// out.  block0: the first G1 block of the batch this kernel runs.
+template <class G>
+__global__ void __launch_bounds__(128, 3) k_batch_exp_rest(const __grid_constant__ VecBatch batch, uint32_t block0, uint32_t in_compressed,
+                                                           const uint32_t* table, uint32_t check, uint32_t* jac_out, uint32_t* status) {
+  extern __shared__ __align__(16) unsigned char tree_raw[];
+  block_batch_exp<G>(block0 + blockIdx.x, batch, in_compressed, table, check, jac_out, status, reinterpret_cast<typename G::F::T*>(tree_raw));
 }
 template <class G1, class G2>
 __global__ void __launch_bounds__(128, 1) k_normalize_chunk(const __grid_constant__ VecBatch b1, const __grid_constant__ VecBatch b2,
@@ -225,8 +237,30 @@ inline int run_batch_exp_chunk(Ctx& c, int si, const VecBatch& b1, const VecBatc
     }
   }
   if (!coop) {
+    uint32_t rest = 0;                                  // G1 blocks left to k_batch_exp_rest (12-limb G1 bodies only)
+    if constexpr (G1::F::L <= 12) {
+      int dev = 0, nsm = 0;
+      CUDA_TRY(cudaGetDevice(&dev));
+      CUDA_TRY(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev));
+      const uint32_t s2 = 2 * (uint32_t)nsm, s3 = 3 * (uint32_t)nsm;   // resident blocks: fused launch, G1-only kernel
+      // the fused launch keeps the G1 blocks that fill the slots its last G2 wave leaves free (a G2 block takes as long as ~2.5 G1
+      // blocks); the rest go to the G1-only kernel in whole waves
+      const uint32_t gap = nb2 % s2 ? s2 - nb2 % s2 : 0, fill = gap * 5 / 2;
+      rest = nb1 > fill ? (nb1 - fill) / s3 * s3 : 0;
+    }
+    const int sj = (rest && c.s[1] && !c.aliased) ? 1 : si;
+    // one profiled span for both kernels: they do the chunk's batch_exp together
     c.begin(PK_BATCH_EXP_CHUNK, si, n1 + n2);
-    k_batch_exp_chunk<G1, G2><<<nb1 + nb2, EXP_BLOCK, TREE_BYTES, st>>>(b1, b2, nb2, in_compressed, d_table, check, d_jac1, d_jac2, d_status);
+    if (sj != si && (rc = c.fork(si, sj))) return rc;
+    if (nb1 - rest + nb2)                               // none when a G2-less batch fills whole waves of the G1-only kernel
+      k_batch_exp_chunk<G1, G2><<<nb1 - rest + nb2, EXP_BLOCK, TREE_BYTES, st>>>(b1, b2, nb2, in_compressed, d_table, check, d_jac1, d_jac2,
+                                                                                 d_status);
+    if constexpr (G1::F::L <= 12) if (rest) {
+      constexpr size_t TREE1 = 16 + 2 * EXP_BLOCK * sizeof(typename G1::F::T);
+      static_assert(TREE1 <= 48 * 1024, "default dynamic shared memory");
+      k_batch_exp_rest<G1><<<rest, EXP_BLOCK, TREE1, c.s[sj]>>>(b1, nb1 - rest, in_compressed, d_table, check, d_jac1, d_status);
+    }
+    if (sj != si && (rc = c.fork(sj, si))) return rc;
     c.end(si);
   }
 #endif
